@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (sm_100a kernels via the C ABI)
   python bench.py --impl reference [--gpus N] [--steps K] ...    # CPU arm: the oracle port on host cores
+  python bench.py ... --dump-outputs DIR                         # also write the timed loop's results as DIR/*.npy
 
 A "step" is ONE Lloyd iteration over this rank's resident partition: fused assign+partial-sum pass over X,
 fixed-order partial reduce, NCCL allreduce of the [k*d sums | k counts | cost] buffer (N>1), finalize.
@@ -67,7 +68,9 @@ TF32_PEAK_TFLOPS = 3666.0 * 148 * 1.965e9 / 1e12
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="Lloyd iterations of each timed region of the headline loop (the cfg3 sub-record and the "
+                         "power-capped run have their own --cfg3-steps / --long-steps)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="cfg2", choices=sorted(CONFIGS))
@@ -86,7 +89,22 @@ def parse_args():
     ap.add_argument("--cfg3-steps", type=int, default=20)
     ap.add_argument("--long-steps", type=int, default=200, help="second timed loop for the power-capped regime (0 = skip)")
     ap.add_argument("--cpu-sample-rows", type=int, default=1_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed Lloyd loops returned in their last step as "
+                         "DIR/<name>.npy (float32 / float64), so that two builds can be compared output for output: "
+                         "the headline loop after --steps iterations, cfg3_* after --cfg3-steps")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy; the inputs are seeded, so the same arguments give the same inputs."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def measured_peaks():
@@ -205,7 +223,7 @@ def cpu_sample(n_rows: int, d: int, k: int, seed: int = 1234):
 
 def cpu_oracle_run(n_rows: int, d: int, k: int, iters: int, threads: int, repeats: int = 3, seed: int = 1234):
     """Times the oracle's C/OpenMP Lloyd port (oracle/kmeans_oracle.c) on a bounded sample: explicit thread count,
-    pages first-touched by the threads that read them, best of `repeats`."""
+    pages first-touched by the threads that read them, best of `repeats`.  Also returns the last run's result."""
     from oracle import c_oracle
 
     c_oracle.set_threads(threads)
@@ -219,7 +237,7 @@ def cpu_oracle_run(n_rows: int, d: int, k: int, iters: int, threads: int, repeat
         dt = time.perf_counter() - t0
         assert out["n_iter"] == iters
         best = dt if best is None else min(best, dt)
-    return n_rows * iters / best, best, c_oracle.num_threads()
+    return n_rows * iters / best, best, c_oracle.num_threads(), out
 
 
 def cpu_sklearn_legs(n_rows: int, d: int, k: int, iters: int, seed: int = 1234):
@@ -264,7 +282,9 @@ def run_reference(args):
     rows = args.cpu_sample_rows
     threads = host_cores()
     cpu_oracle_run(rows, d, k, max(1, min(args.warmup, 2)), threads, repeats=1)
-    val, dt, used = cpu_oracle_run(rows, d, k, args.steps, threads, repeats=3)
+    val, dt, used, out = cpu_oracle_run(rows, d, k, args.steps, threads, repeats=3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"cluster_centers": out["centers"], "inertia": out["inertia"]})
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
@@ -461,6 +481,8 @@ def ingest_record(torch, ctx, dev):
 
 
 def main():
+    # the benchmark leaves the tree it runs from as it found it: no bytecode caches of the modules it imports either
+    sys.dont_write_bytecode = True
     args = parse_args()
     if args.impl == "reference":
         run_reference(args)
@@ -523,7 +545,11 @@ def main():
     X, centers_true = make_blobs_device(torch, dev, n_local, d, k, rank)
     C0, init_mode = pick_init(args.init, args.config, X, centers_true, k, d)
     ctx.kmeans_lloyd(X, C0.clone(), max(args.warmup, 3), -1.0)          # warm-up
-    (ms, st, clocks, shift, _), rep_ms = timed_lloyd_median(torch, dist, ctx, X, C0, args.steps, dev, world, local_rank)
+    (ms, st, clocks, shift, C_out), rep_ms = timed_lloyd_median(torch, dist, ctx, X, C0, args.steps, dev, world,
+                                                                local_rank)
+    # every timed region starts from C0, so these are the centres after exactly --steps Lloyd iterations
+    outputs = {"cluster_centers": C_out.cpu().numpy(), "shift": shift}
+    del C_out
     launches = int(st["kernel_launches"])
     path = {1: "generic", 2: "tcgen05"}.get(st["last_path"], "?")
     value = n_total * args.steps / (ms / 1e3)
@@ -670,8 +696,11 @@ def main():
             torch.cuda.synchronize(dev)
             t_init = time.perf_counter() - t_init0
             ctx.kmeans_lloyd(X3, C03.clone(), 3, -1.0)
-            (ms3, st3, clocks3, shift3, _), rep3 = timed_lloyd_median(torch, dist, ctx, X3, C03, args.cfg3_steps, dev, world,
-                                                                      local_rank)
+            (ms3, st3, clocks3, shift3, C3_out), rep3 = timed_lloyd_median(torch, dist, ctx, X3, C03, args.cfg3_steps, dev,
+                                                                           world, local_rank)
+            outputs["cfg3_cluster_centers"] = C3_out.cpu().numpy()
+            outputs["cfg3_shift"] = shift3
+            del C3_out
             cfg3 = {"value": n3 * world * args.cfg3_steps / (ms3 / 1e3), "unit": UNIT, "n_gpus": world,
                     "steps": args.cfg3_steps, "warmup": 3, "ms_per_step": ms3 / args.cfg3_steps,
                     "repeat_ms_per_step": rep3,
@@ -690,7 +719,7 @@ def main():
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         rows, cpu_iters = args.cpu_sample_rows, 10
         threads = host_cores()
-        val, dt, used = cpu_oracle_run(rows, d, k, cpu_iters, threads, repeats=3)
+        val, dt, used, _ = cpu_oracle_run(rows, d, k, cpu_iters, threads, repeats=3)
         cpu_baseline = {"value": val, "unit": UNIT, "cores": used, "kind": "port",
                         "sample": f"{rows} rows x {cpu_iters} Lloyd iterations of the same blobs shape (k={k}, d={d}), "
                                   f"oracle/kmeans_oracle.c OpenMP fp64, {used} threads set explicitly = {_HOST_CORES_NOTE}, "
@@ -714,6 +743,8 @@ def main():
             "cfg3": cfg3, "parity": parity, "clocks": clocks, "gpu_launches": launches, "final_shift": shift,
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     cc.__exit__(None, None, None)
     if world > 1:
         dist.destroy_process_group()

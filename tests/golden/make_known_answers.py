@@ -35,7 +35,7 @@ def write_lloyd_golden() -> None:
     cases = [
         # name, n, d, k, generator, max_iter, tol
         ("blobs_small", 4096, 16, 8, "blobs", 30, 1e-4),
-        ("blobs_d128_k64", 4096, 128, 64, "blobs", 12, 1e-4),
+        ("blobs_d128_k64", 1536, 128, 64, "blobs", 12, 1e-4),   # X barely compresses: 1536 rows keep the file < 1 MB
         ("uniform_d32_k8", 6000, 32, 8, "uniform", 8, 0.0),
         ("ragged_d20_k5", 1000, 20, 5, "blobs", 20, 1e-4),
     ]
