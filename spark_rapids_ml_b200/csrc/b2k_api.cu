@@ -135,6 +135,8 @@ extern "C" int b2k_reset_stats(b2k_ctx* ctx) {
   return B2K_OK;
 }
 
+// Grows ctx->scratch to at least `bytes`.  Growing frees the old allocation, so no pointer carved before a reserve is
+// used after it: each scratch user reserves for its whole layout first and carves afterwards.
 int b2k_scratch_reserve(b2k_ctx* ctx, size_t bytes) {
   if (bytes <= ctx->scratch_bytes) return B2K_OK;
   if (ctx->scratch) {
@@ -155,21 +157,17 @@ int b2k_scratch_reserve(b2k_ctx* ctx, size_t bytes) {
 }
 
 namespace {
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-// Bump allocator over ctx->scratch.
-struct Arena {
-  char* base;
-  size_t off = 0;
-  explicit Arena(void* b) : base(static_cast<char*>(b)) {}
-  template <typename T>
-  T* take(size_t count) {
-    off = align_up(off, 256);
-    T* p = reinterpret_cast<T*>(base + off);
-    off += count * sizeof(T);
-    return p;
-  }
-};
+// Runs `layout` (int(Arena&): takes every buffer of one scratch user) on a measuring arena, reserves what it took, then
+// runs it again on the scratch to carve the pointers.
+template <typename Layout>
+int carve_scratch(b2k_ctx* ctx, Layout&& layout) {
+  Arena m;
+  B2K_TRY(layout(m));
+  B2K_TRY(b2k_scratch_reserve(ctx, m.off));
+  Arena A(ctx->scratch, ctx->scratch_bytes);
+  B2K_TRY(layout(A));
+  return A.overflow ? b2k_fail(ctx, B2K_ERR_STATE, "scratch layout outgrew its reserve") : B2K_OK;
+}
 
 int check_shape(b2k_ctx* ctx, const char* who, const void* X, int64_t n, int d, int k) {
   if (!ctx) return b2k_fail(nullptr, B2K_ERR_INVALID, std::string(who) + ": ctx is NULL");
@@ -178,11 +176,12 @@ int check_shape(b2k_ctx* ctx, const char* who, const void* X, int64_t n, int d, 
   return B2K_OK;
 }
 
-bool want_fused(b2k_ctx* ctx, int64_t n, int d, int k, const float* X, int* status) {
+// `path`: the kernel path the pass honours (B2K_PATH_*)
+bool want_fused(b2k_ctx* ctx, int path, int64_t n, int d, int k, const float* X, int* status) {
   *status = B2K_OK;
   bool ok = b2k_fused_supported(ctx, n, d, k, X);
-  if (ctx->kernel_path == B2K_PATH_GENERIC) return false;
-  if (ctx->kernel_path == B2K_PATH_TCGEN05 && !ok) {
+  if (path == B2K_PATH_GENERIC) return false;
+  if (path == B2K_PATH_TCGEN05 && !ok) {
     *status = b2k_fail(ctx, B2K_ERR_UNSUPPORTED,
                        "kernel_path=tcgen05 requested but shape (n=" + std::to_string(n) + ", d=" +
                            std::to_string(d) + ", k=" + std::to_string(k) +
@@ -192,7 +191,7 @@ bool want_fused(b2k_ctx* ctx, int64_t n, int d, int k, const float* X, int* stat
   return ok;
 }
 
-// Scratch footprint of one assign/lloyd call.
+// Scratch of one Lloyd loop.
 struct LoopBuffers {
   B2kLoopState* st;
   double* R;
@@ -205,7 +204,6 @@ struct LoopBuffers {
   int P;
   // fused
   B2kFusedPlan plan;
-  void* plan_scratch;
 };
 
 }  // namespace
@@ -224,37 +222,28 @@ namespace {
 struct ChunkedAssign {
   B2kFusedPlan plan;
   int ch = 0;                // chunk size
-  void* ps = nullptr;        // plan scratch
   int32_t* tmp_lab = nullptr;
   float* tmp_md = nullptr;
   int32_t* lab_acc = nullptr;   // used when the caller passes no labels / mindist buffer
   float* md_acc = nullptr;
 };
-// chunk size, 0 = this (d, k) is not chunked
-int chunked_assign_ch(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X) {
-  if (ctx->kernel_path == B2K_PATH_GENERIC || n <= 0 || d > 256) return 0;
+// chunk size, 0 = this (d, k) is not chunked.  `path`: the kernel path the pass honours; `near_tie`: the caller expects
+// near-ties (prefer exact 128-centre chunks, d <= 128).
+int chunked_assign_ch(const b2k_ctx* ctx, int path, bool near_tie, int64_t n, int d, int k, const float* X) {
+  if (path == B2K_PATH_GENERIC || n <= 0 || d > 256) return 0;
   const int ch = (d <= 128 && !ctx->force_variant_t) ? 128 : 256;
-  const bool want = k > 256 || (ch == 128 && k > 128 && ctx->near_tie_hint);
+  const bool want = k > 256 || (ch == 128 && k > 128 && near_tie);
   if (!want || !b2k_fused_supported(ctx, n, d, ch, X)) return 0;
   return ch;
 }
-size_t chunked_assign_bytes(b2k_ctx* ctx, int64_t n, int d, int ch) {
-  B2kFusedPlan plan;
-  if (b2k_fused_plan(ctx, n, d, ch, &plan) != B2K_OK) return 0;
-  return align_up(plan.scratch_bytes, 1024) + 4 * align_up((size_t)n * 4, 256) + 4096;
-}
-// `base`: 1 KB aligned scratch of chunked_assign_bytes(); the caller runs b2k_fused_prepare(ca.plan, ca.ps, ..., ca.ch)
-int chunked_assign_setup(b2k_ctx* ctx, int64_t n, int d, int ch, void* base, ChunkedAssign* ca) {
+// the caller runs b2k_fused_prepare(ca.plan, ...) before chunked_assign_run
+int chunked_assign_layout(b2k_ctx* ctx, int64_t n, int d, int ch, Arena& A, ChunkedAssign* ca) {
   ca->ch = ch;
-  B2K_TRY(b2k_fused_plan(ctx, n, d, ch, &ca->plan));
-  Arena A(base);
   ca->tmp_lab = A.take<int32_t>(n);
   ca->tmp_md = A.take<float>(n);
   ca->lab_acc = A.take<int32_t>(n);
   ca->md_acc = A.take<float>(n);
-  A.off = align_up(A.off, 1024);
-  ca->ps = A.base + A.off;
-  return B2K_OK;
+  return b2k_fused_plan(ctx, n, d, ch, A, &ca->plan);
 }
 int chunked_assign_run(b2k_ctx* ctx, const ChunkedAssign& ca, const float* X, int64_t n, int d, const float* C, int k,
                        int32_t* labels, float* mindist, const B2kLoopState* st, cudaStream_t s) {
@@ -263,8 +252,9 @@ int chunked_assign_run(b2k_ctx* ctx, const ChunkedAssign& ca, const float* X, in
   for (int c0 = 0; c0 < k; c0 += ca.ch) {
     const int base = std::min(c0, k - ca.ch);
     const bool first = c0 == 0;
-    B2K_TRY(b2k_launch_fused(ctx, ca.plan, ca.ps, X, n, d, C + (size_t)base * d, ca.ch, first ? lab : ca.tmp_lab,
-                             first ? md : ca.tmp_md, false, st, s));
+    // every chunk writes mindist, which makes both variants compute the cost: the merge needs no cost partials
+    B2K_TRY(b2k_launch_fused(ctx, ca.plan, X, n, d, C + (size_t)base * d, ca.ch, first ? lab : ca.tmp_lab,
+                             first ? md : ca.tmp_md, false, false, st, s));
     if (!first) B2K_TRY(b2k_launch_merge_chunk(ctx, md, lab, ca.tmp_md, ca.tmp_lab, base, n, st, s));
   }
   return B2K_OK;
@@ -274,56 +264,47 @@ int chunked_assign_run(b2k_ctx* ctx, const ChunkedAssign& ca, const float* X, in
 // ------------------------------------------------------------------------------------------------
 // Lloyd loop
 // ------------------------------------------------------------------------------------------------
+// `norms`: the fit's row-norm scope (null for a standalone call); *path_out: the path the loop ended on (B2K_PATH_*)
 static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, float* C, int max_iter, double tol,
-                      int* n_iter_out, double* shift_out, cudaStream_t s) {
+                      B2kNormScope* norms, int* n_iter_out, double* shift_out, int* path_out, cudaStream_t s) {
   if (max_iter < 0) return b2k_fail(ctx, B2K_ERR_INVALID, "lloyd: max_iter < 0");
   const bool dbg = std::getenv("B2K_DEBUG_TIMING") != nullptr;
   const auto t_entry = std::chrono::steady_clock::now();
   auto since = [&](std::chrono::steady_clock::time_point t0) {
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   };
+  const int path = ctx->kernel_path;
   // k > 256 (d <= 256): the assignment runs in 256-centre chunks on the large-shape kernel, the update stays generic
-  const int chunk_ch = k > 256 ? chunked_assign_ch(ctx, n, d, k, X) : 0;
+  const int chunk_ch = k > 256 ? chunked_assign_ch(ctx, path, false, n, d, k, X) : 0;
   const bool chunked = chunk_ch != 0;
   int st_rc = B2K_OK;
-  const bool fused = chunked ? false : want_fused(ctx, n, d, k, X, &st_rc);
+  const bool fused = chunked ? false : want_fused(ctx, path, n, d, k, X, &st_rc);
   B2K_TRY(st_rc);
   ctx->stats.last_path = (fused || chunked) ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
 
   LoopBuffers B{};
-  size_t gen_bytes = 0;
-  if (fused) B2K_TRY(b2k_fused_plan(ctx, n, d, k, &B.plan));
-  // The large-shape kernel (1xTF32 screening) hands near-tie rows to an exact fix-up; on data where most rows are
-  // near-ties (e.g. uniform noise in 256 dimensions) the generic kernels are several times faster, so the loop may
-  // switch to them between bursts.  The choice is local to the rank: both paths fill the same R buffer.
-  const bool can_switch = fused && B.plan.variant == 1 && ctx->adaptive_path && ctx->kernel_path == B2K_PATH_AUTO;
-  const bool need_generic = !fused || can_switch;
-  if (need_generic) gen_bytes = b2k_update_generic_scratch(ctx, n, d, k, &B.P);
-  const size_t rlen = b2k_reduced_len(k, d);
-  size_t total = 4096 + align_up(rlen * 8, 256) + align_up((size_t)k * 8, 256) + align_up((size_t)k * 4, 256) +
-                 (fused ? align_up(B.plan.scratch_bytes, 1024) + 2048 : 0) +
-                 (need_generic ? align_up((size_t)n * 4, 256) + align_up(gen_bytes, 256) + 4096 : 0) +
-                 (chunked ? chunked_assign_bytes(ctx, n, d, chunk_ch) + 2048 : 0);
-  B2K_TRY(b2k_scratch_reserve(ctx, total));
-  Arena A(ctx->scratch);
-  B.st = A.take<B2kLoopState>(1);
-  B.R = A.take<double>(rlen);
-  B.shift_scratch = A.take<double>(k);
-  B.cnorm = A.take<float>(k);
-  if (need_generic) {
-    B.labels = A.take<int32_t>(n > 0 ? n : 1);
-    B.partials = A.take<float>((size_t)B.P * k * d);
-    B.counts = A.take<int32_t>((size_t)B.P * k);
-  }
-  if (fused) {
-    A.off = align_up(A.off, 1024);
-    B.plan_scratch = A.base + A.off;
-  }
   ChunkedAssign ca;
-  if (chunked) {
-    A.off = align_up(A.off, 1024);
-    B2K_TRY(chunked_assign_setup(ctx, n, d, chunk_ch, A.base + A.off, &ca));
-  }
+  bool can_switch = false;
+  const size_t rlen = b2k_reduced_len(k, d);
+  B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+    B.st = A.take<B2kLoopState>(1);
+    B.R = A.take<double>(rlen);
+    B.shift_scratch = A.take<double>(k);
+    B.cnorm = A.take<float>(k);
+    if (fused) B2K_TRY(b2k_fused_plan(ctx, n, d, k, A, &B.plan));
+    // The large-shape kernel (1xTF32 screening) hands near-tie rows to an exact fix-up; on data where most rows are
+    // near-ties (e.g. uniform noise in 256 dimensions) the generic kernels are several times faster, so the loop may
+    // switch to them between bursts.  The choice is local to the rank: both paths fill the same R buffer.
+    can_switch = fused && B.plan.variant == 1 && ctx->adaptive_path && path == B2K_PATH_AUTO;
+    if (!fused || can_switch) {
+      b2k_update_generic_scratch(ctx, n, d, k, &B.P);
+      B.labels = A.take<int32_t>(n > 0 ? n : 1);
+      B.partials = A.take<float>((size_t)B.P * k * d);
+      B.counts = A.take<int32_t>((size_t)B.P * k);
+    }
+    if (chunked) B2K_TRY(chunked_assign_layout(ctx, n, d, chunk_ch, A, &ca));
+    return B2K_OK;
+  }));
 
   B2kLoopState init{};
   init.iter = 0;
@@ -352,8 +333,8 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
   }
   B2K_CUDA_OK(ctx, cudaEventCreateWithFlags(&poll_ev[0], cudaEventDisableTiming));
   B2K_CUDA_OK(ctx, cudaEventCreateWithFlags(&poll_ev[1], cudaEventDisableTiming));
-  if (fused && max_iter > 0) B2K_TRY(b2k_fused_prepare(ctx, B.plan, B.plan_scratch, X, n, d, k, s));
-  if (chunked && max_iter > 0) B2K_TRY(b2k_fused_prepare(ctx, ca.plan, ca.ps, X, n, d, chunk_ch, s));
+  if (fused && max_iter > 0) B2K_TRY(b2k_fused_prepare(ctx, B.plan, X, n, d, norms, s));
+  if (chunked && max_iter > 0) B2K_TRY(b2k_fused_prepare(ctx, ca.plan, X, n, d, norms, s));
   if (ctx->time_kernels) B2K_CUDA_OK(ctx, cudaEventRecord(loop0, s));
   const double t_setup = since(t_entry);
   const auto t_loop = std::chrono::steady_clock::now();
@@ -377,14 +358,11 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
       if (fused_now) {
         if (e) B2K_CUDA_OK(ctx, cudaEventRecord(e[0], s));
         // cluster sizes of the previous iteration (R = [k*d sums | k counts | cost]) drive the update-warp balancing
-        B2K_TRY(b2k_launch_fused(ctx, B.plan, B.plan_scratch, X, n, d, C, k, nullptr, nullptr, true, B.st, s,
+        B2K_TRY(b2k_launch_fused(ctx, B.plan, X, n, d, C, k, nullptr, nullptr, true, false, B.st, s,
                                  launched > 0 ? B.R + (size_t)k * d : nullptr));
         if (e) B2K_CUDA_OK(ctx, cudaEventRecord(e[1], s));
-        float* partials;
-        int32_t* counts;
-        double* cost_partials;
-        b2k_fused_views(B.plan, B.plan_scratch, n, k, d, &partials, &counts, &cost_partials);
-        B2K_TRY(b2k_launch_reduce_partials(ctx, partials, counts, cost_partials, B.plan.P, B.plan.Pc, k, d, B.R, B.st, s));
+        B2K_TRY(b2k_launch_reduce_partials(ctx, B.plan.partials, B.plan.counts, B.plan.cost_partials, B.plan.P,
+                                           B.plan.Pc, k, d, B.R, B.st, s));
       } else {
         if (e) B2K_CUDA_OK(ctx, cudaEventRecord(e[0], s));
         if (chunked) {
@@ -468,11 +446,11 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
     cudaEventDestroy(loop1);
   }
   ctx->stats.last_n_iter = ctx->h_state->iter;
-  ctx->lloyd_switched = (fused && !fused_now) ? 1 : 0;
-  if (ctx->lloyd_switched) ctx->stats.last_path = B2K_PATH_GENERIC;
+  ctx->stats.last_path = (fused_now || chunked) ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
+  if (path_out) *path_out = ctx->stats.last_path;
   if (fused && ctx->collect_recheck && max_iter > 0) {
     unsigned long long rs[2];
-    B2K_TRY(b2k_fused_recheck_stats(ctx, B.plan, B.plan_scratch, n, k, d, rs, s));
+    B2K_TRY(b2k_fused_recheck_stats(ctx, B.plan, rs, s));
     ctx->stats.recheck_rows = (int64_t)rs[0];
     ctx->stats.recheck_candidates = (int64_t)rs[1];
   }
@@ -486,99 +464,98 @@ extern "C" int b2k_kmeans_lloyd(b2k_ctx* ctx, const float* X, int64_t n_local, i
   B2K_TRY(check_shape(ctx, "b2k_kmeans_lloyd", X, n_local, d, k));
   if (!centers) return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_kmeans_lloyd: centers is NULL");
   B2K_CUDA_OK(ctx, cudaSetDevice(ctx->device));
-  return lloyd_impl(ctx, X, n_local, d, k, centers, max_iter, tol, n_iter_out, shift_out,
+  return lloyd_impl(ctx, X, n_local, d, k, centers, max_iter, tol, nullptr, n_iter_out, shift_out, nullptr,
                     reinterpret_cast<cudaStream_t>(stream));
 }
 
 // ------------------------------------------------------------------------------------------------
-// assign (+ optional total cost): labels/mindist may be NULL.  Scratch beyond `scratch_off` is used.
+// assign (+ optional total cost): labels/mindist may be NULL
 // ------------------------------------------------------------------------------------------------
-static int assign_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, const float* C, int k, int32_t* labels,
-                       float* mindist, double* cost_dev /* device, 1 double, may be NULL */, size_t scratch_off,
-                       cudaStream_t s) {
-  if (const int ch = chunked_assign_ch(ctx, n, d, k, X)) {   // chunks of ch centres through a fused assign pass each
-    const int nblocks = 1024;
-    const size_t off = align_up(scratch_off, 1024);
-    const size_t cbytes = chunked_assign_bytes(ctx, n, d, ch);
-    size_t need = off + cbytes + align_up((size_t)nblocks * 8, 256) + 1024;
-    if (need > ctx->scratch_bytes && scratch_off != 0)
-      return b2k_fail(ctx, B2K_ERR_STATE, "assign_impl: scratch must be pre-reserved by the caller");
-    B2K_TRY(b2k_scratch_reserve(ctx, need));
-    char* base = static_cast<char*>(ctx->scratch) + off;
-    ChunkedAssign ca;
-    B2K_TRY(chunked_assign_setup(ctx, n, d, ch, base, &ca));
-    double* blocks = reinterpret_cast<double*>(base + cbytes);
-    B2K_TRY(b2k_fused_prepare(ctx, ca.plan, ca.ps, X, n, d, ch, s));
-    B2K_TRY(chunked_assign_run(ctx, ca, X, n, d, C, k, labels, mindist, nullptr, s));
-    if (cost_dev) B2K_TRY(b2k_launch_sum_f32_to_f64(ctx, mindist ? mindist : ca.md_acc, n, cost_dev, blocks, nblocks, s));
-    ctx->stats.last_path = B2K_PATH_TCGEN05;
-    if (ctx->collect_recheck) {
-      unsigned long long rs[2];
-      B2K_TRY(b2k_fused_recheck_stats(ctx, ca.plan, ca.ps, n, ch, d, rs, s));
-      ctx->stats.recheck_rows = (int64_t)rs[0];
-      ctx->stats.recheck_candidates = (int64_t)rs[1];
-    }
+namespace {
+// per-call choices of an assign pass
+struct PassOpts {
+  int path;                        // kernel path to honour (B2K_PATH_*): the option, or the path a fit's Lloyd loop ended on
+  bool near_tie = false;           // the caller expects near-ties (chunked_assign_ch)
+  B2kNormScope* norms = nullptr;   // the fit's row-norm scope, for passes over the fit's X
+};
+
+constexpr int kCostBlocks = 1024;   // block sums of a cost formed from mindist
+
+// One assign pass: chunked (ch > 0), one fused pass, or the generic kernels, and the scratch that route takes.
+struct AssignPass {
+  int ch = 0;
+  bool fused = false;
+  ChunkedAssign ca;
+  B2kFusedPlan plan;
+  float* cnorm = nullptr;    // generic
+  float* md = nullptr;       // generic: mindist of its own, for a cost without the caller's mindist
+  double* blocks = nullptr;  // chunked / generic: cost block sums
+};
+
+int assign_layout(b2k_ctx* ctx, const PassOpts& o, const float* X, int64_t n, int d, int k, bool own_md, Arena& A,
+                  AssignPass* p) {
+  if ((p->ch = chunked_assign_ch(ctx, o.path, o.near_tie, n, d, k, X))) {
+    B2K_TRY(chunked_assign_layout(ctx, n, d, p->ch, A, &p->ca));
+    p->blocks = A.take<double>(kCostBlocks);
     return B2K_OK;
   }
-  int st_rc;
-  const bool fused = want_fused(ctx, n, d, k, X, &st_rc);
-  B2K_TRY(st_rc);
-  ctx->stats.last_path = fused ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
-  if (fused) {
-    B2kFusedPlan plan;
-    B2K_TRY(b2k_fused_plan(ctx, n, d, k, &plan));
-    size_t need = align_up(scratch_off, 1024) + align_up(plan.scratch_bytes, 1024) + 1024;
-    if (need > ctx->scratch_bytes && scratch_off != 0)
-      return b2k_fail(ctx, B2K_ERR_STATE, "assign_impl: scratch must be pre-reserved by the caller");
-    B2K_TRY(b2k_scratch_reserve(ctx, need));
-    void* ps = static_cast<char*>(ctx->scratch) + align_up(scratch_off, 1024);
-    B2K_TRY(b2k_fused_prepare(ctx, plan, ps, X, n, d, k, s));
-    ctx->want_cost = cost_dev != nullptr ? 1 : 0;
-    B2K_TRY(b2k_launch_fused(ctx, plan, ps, X, n, d, C, k, labels, mindist, false, nullptr, s));
-    if (cost_dev) {
-      float* partials;
-      int32_t* counts;
-      double* cost_partials;
-      b2k_fused_views(plan, ps, n, k, d, &partials, &counts, &cost_partials);
-      // fold the per-CTA cost partials in index order
-      B2K_TRY(b2k_launch_fold_f64(ctx, cost_partials, plan.Pc, cost_dev, s));
-    }
-    if (ctx->collect_recheck) {
-      unsigned long long rs[2];
-      B2K_TRY(b2k_fused_recheck_stats(ctx, plan, ps, n, k, d, rs, s));
-      ctx->stats.recheck_rows = (int64_t)rs[0];
-      ctx->stats.recheck_candidates = (int64_t)rs[1];
-    }
-  } else {
-    const int nblocks = 1024;
-    size_t need = align_up(scratch_off, 256) + align_up((size_t)k * 4, 256) +
-                  (cost_dev && !mindist ? align_up((size_t)(n > 0 ? n : 1) * 4, 256) : 0) +
-                  align_up((size_t)nblocks * 8, 256) + 1024;
-    if (need > ctx->scratch_bytes && scratch_off != 0)
-      return b2k_fail(ctx, B2K_ERR_STATE, "assign_impl: scratch must be pre-reserved by the caller");
-    B2K_TRY(b2k_scratch_reserve(ctx, need));
-    Arena A(ctx->scratch);
-    A.off = scratch_off;
-    float* cnorm = A.take<float>(k);
-    float* md = mindist;
-    if (cost_dev && !md) md = A.take<float>(n > 0 ? n : 1);
-    double* blocks = A.take<double>(nblocks);
-    B2K_TRY(b2k_launch_center_norms(ctx, C, k, d, cnorm, nullptr, s));
-    B2K_TRY(b2k_launch_assign_generic(ctx, X, n, d, C, cnorm, k, labels, md, nullptr, s));
-    if (cost_dev) B2K_TRY(b2k_launch_sum_f32_to_f64(ctx, md, n, cost_dev, blocks, nblocks, s));
-  }
+  int rc;
+  p->fused = want_fused(ctx, o.path, n, d, k, X, &rc);
+  B2K_TRY(rc);
+  if (p->fused) return b2k_fused_plan(ctx, n, d, k, A, &p->plan);
+  p->cnorm = A.take<float>(k);
+  if (own_md) p->md = A.take<float>(n > 0 ? n : 1);
+  p->blocks = A.take<double>(kCostBlocks);
   return B2K_OK;
 }
 
-// upper bound of what assign_impl needs past scratch_off
-static size_t assign_scratch_bound(b2k_ctx* ctx, int64_t n, int d, int k, const float* X) {
-  size_t b = align_up((size_t)k * 4, 256) + align_up((size_t)(n > 0 ? n : 1) * 4, 256) + 1024 * 8 + 4096;
-  if (const int ch = chunked_assign_ch(ctx, n, d, k, X)) b = std::max(b, chunked_assign_bytes(ctx, n, d, ch) + 1024 * 8 + 8192);
-  if (b2k_fused_supported(ctx, n, d, k, X) && ctx->kernel_path != B2K_PATH_GENERIC) {
-    B2kFusedPlan plan;
-    if (b2k_fused_plan(ctx, n, d, k, &plan) == B2K_OK) b = std::max(b, align_up(plan.scratch_bytes, 1024) + 4096);
+// Takes room for the largest assign pass over X[n, d] with any centre count in `ks`.  The passes themselves carve from
+// a copy of the arena as it was before this call (assign_impl).
+int assign_room(b2k_ctx* ctx, const PassOpts& o, const float* X, int64_t n, int d, std::initializer_list<int> ks,
+                bool own_md, Arena& A) {
+  Arena end = A;
+  for (int kk : ks) {
+    Arena a = A;
+    AssignPass p;
+    B2K_TRY(assign_layout(ctx, o, X, n, d, kk, own_md, a, &p));
+    if (a.off > end.off) end = a;
   }
-  return b;
+  A = end;
+  return B2K_OK;
+}
+}  // namespace
+
+// `A`: the scratch its caller left for the pass (see assign_room)
+static int assign_impl(b2k_ctx* ctx, Arena A, const PassOpts& o, const float* X, int64_t n, int d, const float* C,
+                       int k, int32_t* labels, float* mindist, double* cost_dev /* device, 1 double, may be NULL */,
+                       cudaStream_t s) {
+  AssignPass p;
+  B2K_TRY(assign_layout(ctx, o, X, n, d, k, cost_dev && !mindist, A, &p));
+  if (A.overflow) return b2k_fail(ctx, B2K_ERR_STATE, "assign_impl: the pass outgrows the scratch reserved for it");
+  ctx->stats.last_path = (p.ch || p.fused) ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
+  if (p.ch) {   // chunks of ch centres through a fused assign pass each
+    B2K_TRY(b2k_fused_prepare(ctx, p.ca.plan, X, n, d, o.norms, s));
+    B2K_TRY(chunked_assign_run(ctx, p.ca, X, n, d, C, k, labels, mindist, nullptr, s));
+    if (cost_dev)
+      B2K_TRY(b2k_launch_sum_f32_to_f64(ctx, mindist ? mindist : p.ca.md_acc, n, cost_dev, p.blocks, kCostBlocks, s));
+  } else if (p.fused) {
+    B2K_TRY(b2k_fused_prepare(ctx, p.plan, X, n, d, o.norms, s));
+    B2K_TRY(b2k_launch_fused(ctx, p.plan, X, n, d, C, k, labels, mindist, false, cost_dev != nullptr, nullptr, s));
+    // fold the per-CTA cost partials in index order
+    if (cost_dev) B2K_TRY(b2k_launch_fold_f64(ctx, p.plan.cost_partials, p.plan.Pc, cost_dev, s));
+  } else {
+    float* md = mindist ? mindist : p.md;
+    B2K_TRY(b2k_launch_center_norms(ctx, C, k, d, p.cnorm, nullptr, s));
+    B2K_TRY(b2k_launch_assign_generic(ctx, X, n, d, C, p.cnorm, k, labels, md, nullptr, s));
+    if (cost_dev) B2K_TRY(b2k_launch_sum_f32_to_f64(ctx, md, n, cost_dev, p.blocks, kCostBlocks, s));
+  }
+  if (ctx->collect_recheck && (p.ch || p.fused)) {
+    unsigned long long rs[2];
+    B2K_TRY(b2k_fused_recheck_stats(ctx, p.ch ? p.ca.plan : p.plan, rs, s));
+    ctx->stats.recheck_rows = (int64_t)rs[0];
+    ctx->stats.recheck_candidates = (int64_t)rs[1];
+  }
+  return B2K_OK;
 }
 
 extern "C" int b2k_kmeans_assign(b2k_ctx* ctx, const float* X, int64_t n, int d, const float* centers, int k,
@@ -587,7 +564,13 @@ extern "C" int b2k_kmeans_assign(b2k_ctx* ctx, const float* X, int64_t n, int d,
   if (!centers) return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_kmeans_assign: centers is NULL");
   if (n == 0) return B2K_OK;
   B2K_CUDA_OK(ctx, cudaSetDevice(ctx->device));
-  return assign_impl(ctx, X, n, d, centers, k, labels_out, mindist_out, nullptr, 0,
+  const PassOpts o{ctx->kernel_path};
+  Arena pass;
+  B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+    pass = A;
+    return assign_room(ctx, o, X, n, d, {k}, false, A);
+  }));
+  return assign_impl(ctx, pass, o, X, n, d, centers, k, labels_out, mindist_out, nullptr,
                      reinterpret_cast<cudaStream_t>(stream));
 }
 
@@ -607,9 +590,12 @@ int gather_sizes(b2k_ctx* ctx, int64_t n_local, Rows* rows, cudaStream_t s) {
   if (ctx->nranks == 1) {
     rows->sizes[0] = n_local;
   } else {
-    B2K_TRY(b2k_scratch_reserve(ctx, 4096 + 16 * (size_t)ctx->nranks));
-    int64_t* send = reinterpret_cast<int64_t*>(ctx->scratch);
-    int64_t* recv = send + 32;
+    int64_t *send, *recv;
+    B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+      send = A.take<int64_t>(1);
+      recv = A.take<int64_t>(ctx->nranks);
+      return B2K_OK;
+    }));
     B2K_CUDA_OK(ctx, cudaMemcpyAsync(send, &n_local, 8, cudaMemcpyHostToDevice, s));
     B2K_TRY(b2k_comm_allgather_i64(ctx, send, recv, 1, s));
     B2K_CUDA_OK(ctx, cudaMemcpyAsync(rows->sizes.data(), recv, 8 * (size_t)ctx->nranks, cudaMemcpyDeviceToHost, s));
@@ -722,20 +708,21 @@ static int init_random(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, ui
     return b2k_fail(ctx, B2K_ERR_INVALID, "init=random: fewer rows (" + std::to_string(rows.total) + ") than k");
   std::mt19937_64 rng(seed);
   std::vector<int64_t> gidx = sample_distinct(rng, rows.total, k);
-  B2K_TRY(b2k_scratch_reserve(ctx, 4096 + (size_t)k * 8));
-  int64_t* idx_dev = reinterpret_cast<int64_t*>(static_cast<char*>(ctx->scratch) + 1024);
+  int64_t* idx_dev;
+  B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+    idx_dev = A.take<int64_t>(k);
+    return B2K_OK;
+  }));
   return fetch_global_rows(ctx, X, n, d, rows, gidx, C, idx_dev, s);
 }
 
 // Scalable k-means++ (k-means||): the reference forwards init="scalable-k-means++", oversampling_factor=2.0
 // (clustering.py:134-136).  Distributional parity only (the reference's own seeded test is xfail).
 static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, uint64_t seed,
-                                double oversampling, float* C, cudaStream_t s) {
-  struct HintGuard {   // the candidate passes are near-tie heavy: see chunked_assign_ch
-    b2k_ctx* c;
-    explicit HintGuard(b2k_ctx* c_) : c(c_) { c->near_tie_hint = 1; }
-    ~HintGuard() { c->near_tie_hint = 0; }
-  } hint_guard(ctx);
+                                double oversampling, B2kNormScope* norms, float* C, cudaStream_t s) {
+  // the candidate passes are near-tie heavy (see chunked_assign_ch); only those over X share the fit's row norms
+  const PassOpts ox{ctx->kernel_path, true, norms};
+  const PassOpts ocand{ctx->kernel_path, true, nullptr};
   const int rounds = 5;
   Rows rows;
   B2K_TRY(gather_sizes(ctx, n, &rows, s));
@@ -744,35 +731,32 @@ static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, 
   const double ell = oversampling * k;
   const int cap = (int)std::min<int64_t>(rows.total, (int64_t)(4 * ell) + 64);  // per-round candidate cap
   const int Mmax = 1 + rounds * cap + k;
-  // scratch (all taken from one arena sized from cap / nranks: no fixed-offset control region):
-  //   idx[cap+8] | n_picked | phi | blocks[1024] | exchange[(cap+1)*(nranks+1)] | mind[n] | dn[n] | labels[n] | lab_new[n] |
-  //   cand[Mmax*d] | newc[cap*d] | hist[Mmax] | assign scratch
-  size_t nn = (size_t)(n > 0 ? n : 1);
+  const size_t nn = (size_t)(n > 0 ? n : 1);
   const size_t per = (size_t)cap + 1;   // [count | cap indices] per rank in the candidate exchange
-  size_t fixed = align_up((size_t)(cap + 8) * 8, 256) + 256 + 256 + align_up(1024 * 8, 256) +
-                 align_up(per * (size_t)(ctx->nranks + 1) * 8, 256) + 4 * align_up(nn * 4, 256) +
-                 align_up((size_t)Mmax * d * 4, 256) + align_up((size_t)cap * d * 4, 256) +
-                 align_up((size_t)Mmax * 8, 256) + 8192;
-  // the assign passes below run with 1 .. Mmax centres: small counts take a fused kernel (its scratch holds per-CTA
-  // partial slots and, for the large-shape kernel, the row norms), large ones the generic path
-  size_t abound = 0;
-  for (int kk : {1, std::min(cap, 128), std::min(cap, 256), cap, Mmax})
-    abound = std::max(abound, assign_scratch_bound(ctx, n, d, kk, X));
-  B2K_TRY(b2k_scratch_reserve(ctx, fixed + abound + 4096));
-  Arena A(ctx->scratch);
-  int64_t* idx_dev = A.take<int64_t>(cap + 8);
-  int* n_picked_dev = A.take<int>(8);
-  double* phi_dev = A.take<double>(4);
-  double* blocks = A.take<double>(1024);
-  int64_t* xchg = A.take<int64_t>(per * (size_t)(ctx->nranks + 1));
-  float* mind = A.take<float>(nn);
-  float* dn = A.take<float>(nn);
-  int32_t* labels = A.take<int32_t>(nn);    // running nearest candidate of every row (global candidate index)
-  int32_t* lab_new = A.take<int32_t>(nn);   // nearest among one round's new candidates
-  float* cand = A.take<float>((size_t)Mmax * d);
-  float* newc = A.take<float>((size_t)cap * d);
-  double* hist = A.take<double>(Mmax);
-  const size_t assign_off = align_up(A.off, 1024);
+  int64_t *idx_dev, *xchg;
+  int* n_picked_dev;
+  double *phi_dev, *blocks, *hist;
+  float *mind, *dn, *cand, *newc;
+  int32_t *labels, *lab_new;
+  Arena pass;
+  B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+    idx_dev = A.take<int64_t>(cap + 8);
+    n_picked_dev = A.take<int>(8);
+    phi_dev = A.take<double>(4);
+    blocks = A.take<double>(1024);
+    xchg = A.take<int64_t>(per * (size_t)(ctx->nranks + 1));
+    mind = A.take<float>(nn);
+    dn = A.take<float>(nn);
+    labels = A.take<int32_t>(nn);    // running nearest candidate of every row (global candidate index)
+    lab_new = A.take<int32_t>(nn);   // nearest among one round's new candidates
+    cand = A.take<float>((size_t)Mmax * d);
+    newc = A.take<float>((size_t)cap * d);
+    hist = A.take<double>(Mmax);
+    pass = A;
+    // the assign passes below run with 1 .. Mmax centres: small counts take a fused kernel (its scratch holds per-CTA
+    // partial slots and, for the large-shape kernel, the row norms), larger ones chunks or the generic path
+    return assign_room(ctx, ox, X, n, d, {1, std::min(cap, 128), std::min(cap, 256), cap, Mmax}, false, A);
+  }));
 
   std::mt19937_64 rng(seed);
   int M = 0;
@@ -781,7 +765,7 @@ static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, 
     std::vector<int64_t> g{U(rng)};
     B2K_TRY(fetch_global_rows(ctx, X, n, d, rows, g, cand, idx_dev, s));
     M = 1;
-    B2K_TRY(assign_impl(ctx, X, n, d, cand, 1, nullptr, mind, phi_dev, assign_off, s));
+    B2K_TRY(assign_impl(ctx, pass, ox, X, n, d, cand, 1, nullptr, mind, phi_dev, s));
     B2K_CUDA_OK(ctx, cudaMemsetAsync(labels, 0, nn * 4, s));   // every row is nearest to candidate 0 so far
   }
   std::vector<int64_t> picked_host(cap);
@@ -843,7 +827,7 @@ static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, 
     // nearest among the new candidates, folded into the running (min distance, nearest candidate): strict '<' keeps the
     // earlier candidate on ties, so after the last round `labels` IS the argmin over all candidates — the k-means||
     // weights need no extra pass over X
-    B2K_TRY(assign_impl(ctx, X, n, d, newc, m, lab_new, dn, nullptr, assign_off, s));
+    B2K_TRY(assign_impl(ctx, pass, ox, X, n, d, newc, m, lab_new, dn, nullptr, s));
     B2K_TRY(b2k_launch_merge_chunk(ctx, mind, labels, dn, lab_new, M, n, nullptr, s));
     M += m;
   }
@@ -851,7 +835,7 @@ static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, 
     std::vector<int64_t> extra = sample_distinct(rng, rows.total, k - M + 1);
     B2K_TRY(fetch_global_rows(ctx, X, n, d, rows, extra, cand + (size_t)M * d, idx_dev, s));
     M += (int)extra.size();
-    B2K_TRY(assign_impl(ctx, X, n, d, cand, M, labels, nullptr, nullptr, assign_off, s));
+    B2K_TRY(assign_impl(ctx, pass, ox, X, n, d, cand, M, labels, nullptr, nullptr, s));
   }
   // weights = #points closest to each candidate (the running argmin of the rounds)
   B2K_TRY(b2k_launch_histogram(ctx, labels, n, M, hist, s));
@@ -866,18 +850,21 @@ static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, 
   // greedy weighted k-means++ on the host (table look-ups), then 10 weighted Lloyd steps on the device: the assignment
   // of the M candidates through the same kernels as any other assign pass, the weighted update in fixed order (fp64)
   std::vector<float> D2h((size_t)M * M);
-  const size_t reg = align_up((size_t)M * d * 4, 256) + align_up((size_t)M * M * 4, 256) + align_up((size_t)M * 8, 256) +
-                     align_up((size_t)k * d * 4, 256) + align_up((size_t)M * 4, 256) + align_up((size_t)k * 8, 256) + 4096;
-  B2K_TRY(b2k_scratch_reserve(ctx, reg + assign_scratch_bound(ctx, M, d, k, static_cast<const float*>(ctx->scratch)) + 4096));
-  // the scratch may have moved: only `cand` is needed from here on, and it was copied to P above
-  Arena R(ctx->scratch);
-  float* candd = R.take<float>((size_t)M * d);
-  float* D2d = R.take<float>((size_t)M * M);
-  double* wts_dev = R.take<double>(M);
-  float* Ck_dev = R.take<float>((size_t)k * d);
-  int32_t* lab_dev = R.take<int32_t>(M);
-  int64_t* chosen_dev = R.take<int64_t>(k);
-  const size_t refine_off = align_up(R.off, 1024);
+  // the scratch may move: only `cand` is needed from here on, and it was copied to P above
+  float *candd, *D2d, *Ck_dev;
+  double* wts_dev;
+  int32_t* lab_dev;
+  int64_t* chosen_dev;
+  B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+    candd = A.take<float>((size_t)M * d);
+    D2d = A.take<float>((size_t)M * M);
+    wts_dev = A.take<double>(M);
+    Ck_dev = A.take<float>((size_t)k * d);
+    lab_dev = A.take<int32_t>(M);
+    chosen_dev = A.take<int64_t>(k);
+    pass = A;
+    return assign_room(ctx, ocand, candd, M, d, {k}, false, A);
+  }));
   B2K_CUDA_OK(ctx, cudaMemcpyAsync(candd, P.data(), P.size() * 4, cudaMemcpyHostToDevice, s));
   B2K_CUDA_OK(ctx, cudaMemcpyAsync(wts_dev, wts.data(), (size_t)M * 8, cudaMemcpyHostToDevice, s));
   B2K_TRY(b2k_launch_pairwise_sqdist(ctx, candd, M, d, D2d, s));
@@ -889,7 +876,7 @@ static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, 
   B2K_CUDA_OK(ctx, cudaStreamSynchronize(s));  // `chosen` is pageable
   B2K_TRY(b2k_launch_gather_rows(ctx, candd, d, chosen_dev, k, Ck_dev, 0, s));
   for (int it = 0; it < 10; ++it) {
-    B2K_TRY(assign_impl(ctx, candd, M, d, Ck_dev, k, lab_dev, nullptr, nullptr, refine_off, s));
+    B2K_TRY(assign_impl(ctx, pass, ocand, candd, M, d, Ck_dev, k, lab_dev, nullptr, nullptr, s));
     B2K_TRY(b2k_launch_weighted_update(ctx, candd, wts_dev, lab_dev, M, d, k, Ck_dev, s));
   }
   B2K_CUDA_OK(ctx, cudaMemcpyAsync(C, Ck_dev, (size_t)k * d * 4, cudaMemcpyDeviceToDevice, s));
@@ -920,19 +907,7 @@ extern "C" int b2k_kmeans_fit(b2k_ctx* ctx, const float* X, int64_t n_local, int
         return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_kmeans_fit: empty partition (rank " + std::to_string(r) +
                                                   " has n_local == 0)");
   }
-  struct NormScope {   // see b2k_ctx::xnorm_scope_X
-    b2k_ctx* c;
-    NormScope(b2k_ctx* c_, const float* X_, int64_t n_, int d_) : c(c_) {
-      c->xnorm_scope_X = X_;
-      c->xnorm_scope_n = n_;
-      c->xnorm_scope_d = d_;
-      c->xnorm_cache_valid = 0;
-    }
-    ~NormScope() {
-      c->xnorm_scope_X = nullptr;
-      c->xnorm_cache_valid = 0;
-    }
-  } norm_scope(ctx, X, n_local, d);
+  B2kNormScope norms{X, n_local};
   switch (init_mode) {
     case B2K_INIT_ARRAY:
       if (!init_centers) return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_kmeans_fit: init_centers is NULL");
@@ -943,22 +918,25 @@ extern "C" int b2k_kmeans_fit(b2k_ctx* ctx, const float* X, int64_t n_local, int
       B2K_TRY(init_random(ctx, X, n_local, d, k, seed, centers_out, s));
       break;
     case B2K_INIT_KMEANS_PARALLEL:
-      B2K_TRY(init_kmeans_parallel(ctx, X, n_local, d, k, seed, oversampling > 0 ? oversampling : 2.0,
+      B2K_TRY(init_kmeans_parallel(ctx, X, n_local, d, k, seed, oversampling > 0 ? oversampling : 2.0, &norms,
                                    centers_out, s));
       break;
     default:
       return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_kmeans_fit: unknown init_mode");
   }
-  B2K_TRY(lloyd_impl(ctx, X, n_local, d, k, centers_out, max_iter, tol, n_iter_out, nullptr, s));
+  int lloyd_path;
+  B2K_TRY(lloyd_impl(ctx, X, n_local, d, k, centers_out, max_iter, tol, &norms, n_iter_out, nullptr, &lloyd_path, s));
   if (inertia_out) {
-    // the inertia pass follows the Lloyd loop's choice of path (see lloyd_impl: adaptive_path)
-    const int saved_path = ctx->kernel_path;
-    if (ctx->lloyd_switched) ctx->kernel_path = B2K_PATH_GENERIC;
-    int rc = b2k_scratch_reserve(ctx, 4096 + assign_scratch_bound(ctx, n_local, d, k, X));
-    double* cost_dev = reinterpret_cast<double*>(ctx->scratch);
-    if (rc == B2K_OK) rc = assign_impl(ctx, X, n_local, d, centers_out, k, nullptr, nullptr, cost_dev, 1024, s);
-    ctx->kernel_path = saved_path;
-    B2K_TRY(rc);
+    // the inertia pass follows the path the Lloyd loop ended on (see lloyd_impl: adaptive_path)
+    const PassOpts o{lloyd_path, false, &norms};
+    double* cost_dev;
+    Arena pass;
+    B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
+      cost_dev = A.take<double>(1);
+      pass = A;
+      return assign_room(ctx, o, X, n_local, d, {k}, true, A);
+    }));
+    B2K_TRY(assign_impl(ctx, pass, o, X, n_local, d, centers_out, k, nullptr, nullptr, cost_dev, s));
     if (ctx->nranks > 1) B2K_TRY(b2k_comm_allreduce_f64(ctx, cost_dev, 1, s));
     B2K_CUDA_OK(ctx, cudaMemcpyAsync(inertia_out, cost_dev, 8, cudaMemcpyDeviceToHost, s));
     B2K_CUDA_OK(ctx, cudaStreamSynchronize(s));

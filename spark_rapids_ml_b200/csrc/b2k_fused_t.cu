@@ -1058,55 +1058,33 @@ __global__ void __launch_bounds__(256) k_fix_accum_t(const FixArgs f) {
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-struct TLayout {
-  size_t off_ct, off_cnorm, off_thr, off_tab, off_rstat, off_partials, off_counts, off_cost, off_xnorm, off_fixlist, off_fixmask,
-      off_fixcnt, total;
-  int npairs, seg_cap, mask_cap;
-};
-TLayout t_layout(const B2kFusedPlan& p, int64_t n, int k, int d) {
-  auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-  TLayout L{};
-  size_t o = 0;
-  L.off_ct = o; o = al(o + (size_t)256 * p.DP * 4);
-  L.off_cnorm = o; o = al(o + 512 * 4);
-  L.off_thr = o; o = al(o + 16);
-  L.off_tab = o; o = al(o + 512);
-  L.off_rstat = o; o = al(o + 16);
-  L.off_partials = o; o = al(o + (size_t)p.P * k * d * 4);
-  L.off_counts = o; o = al(o + (size_t)p.P * k * 4);
-  L.off_cost = o; o = al(o + (size_t)p.Pc * 8);
-  L.off_xnorm = o; o = al(o + (size_t)(n > 0 ? n : 1) * 8);
+void t_layout(B2kFusedPlan* p, int64_t n, int k, int d, Arena& A) {
+  p->ct = A.take<float>((size_t)256 * p->DP, 1024);
+  p->cnorm = A.take<float>(512);
+  p->thr = A.take<float>(4);
+  p->keytab = A.take<uint8_t>(512);
+  p->rstat = A.take<unsigned long long>(2);
+  p->partials = A.take<float>((size_t)p->P * k * d);
+  p->counts = A.take<int32_t>((size_t)p->P * k);
+  p->cost_partials = A.take<double>(p->Pc);
+  p->xnorm = A.take<float2>(n > 0 ? n : 1);
   // deferred-row segments: a pair can defer every row it sees; candidate masks for the first 1/4 of a segment (entries
   // beyond that are decided against every cluster)
-  L.npairs = p.grid / 2;
+  const int npairs = p->grid / 2;
   const int64_t nsteps = (n + TN - 1) / TN;
-  const int64_t nit_max = (nsteps + L.npairs - 1) / L.npairs;
-  L.seg_cap = (int)(nit_max * TN);
-  L.mask_cap = (int)std::min<int64_t>(L.seg_cap, ((nit_max + 3) / 4) * TN);
-  L.off_fixlist = o; o = al(o + (size_t)L.npairs * L.seg_cap * 8);
-  L.off_fixmask = o; o = al(o + (size_t)L.npairs * L.mask_cap * 32);
-  L.off_fixcnt = o; o = al(o + (size_t)L.npairs * 4);
-  L.total = o;
-  return L;
+  const int64_t nit_max = (nsteps + npairs - 1) / npairs;
+  p->seg_cap = (int)(nit_max * TN);
+  p->mask_cap = (int)std::min<int64_t>(p->seg_cap, ((nit_max + 3) / 4) * TN);
+  p->fix_list = A.take<int2>((size_t)npairs * p->seg_cap);
+  p->fix_masks = A.take<uint32_t>((size_t)npairs * p->mask_cap * 8);
+  p->fix_count = A.take<int32_t>(npairs);
 }
 
 template <int NCH, bool UPD>
 int launch_t(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const TArgs& a, cudaStream_t s) {
   auto kern = k_fused_t<NCH, UPD>;
   B2K_CUDA_OK(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(NTHREADS);
-  cfg.dynamicSmemBytes = SMEM_BYTES;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  B2K_CUDA_OK(ctx, cudaLaunchKernelEx(&cfg, kern, mx, a));
+  B2K_TRY(b2k_launch_pair(ctx, kern, grid, NTHREADS, SMEM_BYTES, s, mx, a));
   B2K_CUDA_OK(ctx, cudaGetLastError());
   return B2K_OK;
 }
@@ -1120,7 +1098,7 @@ bool b2k_fused_t_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const fl
   return true;
 }
 
-int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, B2kFusedPlan* plan) {
+int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan) {
   plan->variant = 1;
   plan->KP = 256;
   plan->DP = d <= 128 ? 128 : 256;
@@ -1133,64 +1111,45 @@ int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, B2kFusedPlan* plan) 
   plan->grid = grid;
   plan->P = grid / 2 + FIX_SLOTS;             // one slot per CTA pair + the deferred rows' slots (k_fix_accum_t)
   plan->Pc = grid + 8 * ctx->sm_count;        // cost partials: one per CTA + one per k_fix_labels_t CTA
-  plan->scratch_bytes = t_layout(*plan, n, k, d).total;
+  t_layout(plan, n, k, d, A);
   return B2K_OK;
 }
 
-void b2k_fused_t_views(const B2kFusedPlan& plan, void* plan_scratch, int64_t n, int k, int d, float** partials,
-                       int32_t** counts, double** cost_partials, unsigned long long** rstat) {
-  TLayout L = t_layout(plan, n, k, d);
-  char* b = static_cast<char*>(plan_scratch);
-  *partials = reinterpret_cast<float*>(b + L.off_partials);
-  *counts = reinterpret_cast<int32_t*>(b + L.off_counts);
-  *cost_partials = reinterpret_cast<double*>(b + L.off_cost);
-  if (rstat) *rstat = reinterpret_cast<unsigned long long*>(b + L.off_rstat);
-}
-
-static bool xnorm_in_scope(const b2k_ctx* ctx, const float* X, int64_t n, int d) {
-  return ctx->xnorm_scope_X != nullptr && ctx->xnorm_scope_X == X && ctx->xnorm_scope_n == n && ctx->xnorm_scope_d == d;
-}
-
-// once per fit / lloyd / assign call: row norms of X into the plan scratch (or, inside b2k_kmeans_fit, once per fit into
-// the context's cache); clears the recheck counters
-int b2k_fused_t_prepare(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d,
-                        int k, cudaStream_t s) {
-  TLayout L = t_layout(plan, n, k, d);
-  char* b = static_cast<char*>(plan_scratch);
-  B2K_CUDA_OK(ctx, cudaMemsetAsync(b + L.off_rstat, 0, 16, s));
+// once per fit / lloyd / assign call: row norms of X into the plan scratch (or, with the fit's norm scope, once per fit
+// into the context's cache); clears the recheck counters
+int b2k_fused_t_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
+                        cudaStream_t s) {
+  B2K_CUDA_OK(ctx, cudaMemsetAsync(plan.rstat, 0, 16, s));
   int blocks = ctx->sm_count * 8;
-  float2* dst = reinterpret_cast<float2*>(b + L.off_xnorm);
-  if (xnorm_in_scope(ctx, X, n, d)) {   // inside one b2k_kmeans_fit: one norms pass for all of its passes over X
+  if (norms) {
+    if (norms->X != X || norms->n != n) return b2k_fail(ctx, B2K_ERR_STATE, "fused_t: norm scope of another matrix");
     if (ctx->xnorm_cache_rows < n) {
       if (ctx->xnorm_cache) cudaFree(ctx->xnorm_cache);
       ctx->xnorm_cache = nullptr;
       ctx->xnorm_cache_rows = 0;
       B2K_CUDA_OK(ctx, cudaMalloc(&ctx->xnorm_cache, (size_t)n * sizeof(float2)));
       ctx->xnorm_cache_rows = n;
-      ctx->xnorm_cache_valid = 0;
+      norms->valid = false;
     }
-    if (ctx->xnorm_cache_valid) return B2K_OK;
-    dst = static_cast<float2*>(ctx->xnorm_cache);
-    ctx->xnorm_cache_valid = 1;
+    plan.xnorm = static_cast<float2*>(ctx->xnorm_cache);
+    if (norms->valid) return B2K_OK;
+    norms->valid = true;
   }
-  k_row_norms<<<blocks, 256, 0, s>>>(X, n, d, dst);
+  k_row_norms<<<blocks, 256, 0, s>>>(X, n, d, plan.xnorm);
   ctx->stats.kernel_launches++;
   B2K_CUDA_OK(ctx, cudaGetLastError());
   return B2K_OK;
 }
 
-int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d,
-                       const float* C, int k, int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost,
-                       const B2kLoopState* st, cudaStream_t s, const double* prev_counts) {
-  TLayout L = t_layout(plan, n, k, d);
-  char* b = static_cast<char*>(plan_scratch);
-  float* Ct = reinterpret_cast<float*>(b + L.off_ct);
-  float* cnorm = reinterpret_cast<float*>(b + L.off_cnorm);
-  float* thr = reinterpret_cast<float*>(b + L.off_thr);
-  uint8_t* keytab = reinterpret_cast<uint8_t*>(b + L.off_tab);
+int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int64_t n, int d, const float* C, int k,
+                       int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost, const B2kLoopState* st,
+                       cudaStream_t s, const double* prev_counts) {
+  float* cnorm = plan.cnorm;
+  uint8_t* keytab = plan.keytab;
+  const int npairs = plan.grid / 2;
 
-  k_prep_centers_t<<<32, 256, 0, s>>>(C, k, d, plan.DP, Ct, cnorm, st);
-  k_tables_t<<<1, 256, 0, s>>>(do_update ? prev_counts : nullptr, k, cnorm, keytab, keytab + 256, thr, st);
+  k_prep_centers_t<<<32, 256, 0, s>>>(C, k, d, plan.DP, plan.ct, cnorm, st);
+  k_tables_t<<<1, 256, 0, s>>>(do_update ? prev_counts : nullptr, k, cnorm, keytab, keytab + 256, plan.thr, st);
   ctx->stats.kernel_launches += 2;
   B2K_CUDA_OK(ctx, cudaGetLastError());
 
@@ -1202,17 +1161,16 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratc
   a.nsteps = (int)((n + TN - 1) / TN);
   a.k = k;
   a.d = d;
-  a.Ct = Ct;
+  a.Ct = plan.ct;
   a.C32 = C;
   a.cnorm = cnorm;
-  a.thr = thr;
-  a.xnorm = (xnorm_in_scope(ctx, X, n, d) && ctx->xnorm_cache_valid) ? static_cast<const float2*>(ctx->xnorm_cache)
-                                                                      : reinterpret_cast<const float2*>(b + L.off_xnorm);
+  a.thr = plan.thr;
+  a.xnorm = plan.xnorm;
   a.keytab = keytab;
   a.keyinv = keytab + 256;
-  a.partials = reinterpret_cast<float*>(b + L.off_partials);
-  a.counts = reinterpret_cast<int32_t*>(b + L.off_counts);
-  a.cost_partials = reinterpret_cast<double*>(b + L.off_cost);
+  a.partials = plan.partials;
+  a.counts = plan.counts;
+  a.cost_partials = plan.cost_partials;
   a.labels_out = labels_out;
   a.mind_out = mindist_out;
   a.need_cost = need_cost ? 1 : 0;
@@ -1226,14 +1184,14 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratc
     ctx->prof_grid = 2;
   }
 #endif
-  a.rstat = reinterpret_cast<unsigned long long*>(b + L.off_rstat);
-  a.fix_list = reinterpret_cast<int2*>(b + L.off_fixlist);
-  a.fix_masks = reinterpret_cast<uint32_t*>(b + L.off_fixmask);
-  a.fix_count = reinterpret_cast<int32_t*>(b + L.off_fixcnt);
-  a.seg_cap = L.seg_cap;
-  a.mask_cap = L.mask_cap;
+  a.rstat = plan.rstat;
+  a.fix_list = plan.fix_list;
+  a.fix_masks = plan.fix_masks;
+  a.fix_count = plan.fix_count;
+  a.seg_cap = plan.seg_cap;
+  a.mask_cap = plan.mask_cap;
   a.st = st;
-  if (L.npairs > FIX_MAXP) return b2k_fail(ctx, B2K_ERR_STATE, "fused_t: more CTA pairs than the fix-up kernels index");
+  if (npairs > FIX_MAXP) return b2k_fail(ctx, B2K_ERR_STATE, "fused_t: more CTA pairs than the fix-up kernels index");
 
   int rc;
   if (plan.DP == 128) rc = do_update ? launch_t<4, true>(ctx, plan.grid, mx, a, s) : launch_t<4, false>(ctx, plan.grid, mx, a, s);
@@ -1253,9 +1211,9 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratc
   f.list = a.fix_list;
   f.masks = a.fix_masks;
   f.count = a.fix_count;
-  f.npairs = L.npairs;
-  f.seg_cap = L.seg_cap;
-  f.mask_cap = L.mask_cap;
+  f.npairs = npairs;
+  f.seg_cap = plan.seg_cap;
+  f.mask_cap = plan.mask_cap;
   f.labels_out = labels_out;
   f.mind_out = mindist_out;
   f.need_cost = need_cost ? 1 : 0;

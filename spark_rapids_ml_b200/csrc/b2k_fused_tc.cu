@@ -937,23 +937,8 @@ int launch_inst_nc(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const CUtensor
   using G = Cfg<KP, DP, PAIR>;
   auto kern = k_fused_assign_update<KP, DP, PAIR, NC>;
   B2K_CUDA_OK(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM_BYTES));
-  if constexpr (PAIR) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(NTHREADS);
-    cfg.dynamicSmemBytes = G::SMEM_BYTES;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;   // the CTA pair of tcgen05 cta_group::2
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    B2K_CUDA_OK(ctx, cudaLaunchKernelEx(&cfg, kern, mx, mh, ml, a));
-  } else {
-    kern<<<grid, NTHREADS, G::SMEM_BYTES, s>>>(mx, mh, ml, a);
-  }
+  if constexpr (PAIR) B2K_TRY(b2k_launch_pair(ctx, kern, grid, NTHREADS, G::SMEM_BYTES, s, mx, mh, ml, a));
+  else kern<<<grid, NTHREADS, G::SMEM_BYTES, s>>>(mx, mh, ml, a);
   B2K_CUDA_OK(ctx, cudaGetLastError());
   return B2K_OK;
 }
@@ -965,22 +950,14 @@ int launch_inst(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const CUtensorMap
                      : launch_inst_nc<KP, DP, PAIR, false>(ctx, grid, mx, mh, ml, a, s);
 }
 
-struct PlanLayout {
-  size_t off_chi, off_clo, off_cnorm, off_tab, off_partials, off_counts, off_cost, total;
-};
-PlanLayout plan_layout(const B2kFusedPlan& p, int k, int d) {
-  auto al = [](size_t v) { return (v + 255) / 256 * 256; };
-  PlanLayout L{};
-  size_t o = 0;
-  L.off_chi = o; o = al(o + (size_t)p.KP * p.DP * 4);
-  L.off_clo = o; o = al(o + (size_t)p.KP * p.DP * 4);
-  L.off_cnorm = o; o = al(o + (size_t)p.KP * 4);
-  L.off_tab = o; o = al(o + 512);
-  L.off_partials = o; o = al(o + (size_t)p.grid * k * d * 4);
-  L.off_counts = o; o = al(o + (size_t)p.grid * k * 4);
-  L.off_cost = o; o = al(o + (size_t)p.grid * 8);
-  L.total = o;
-  return L;
+void plan_layout(B2kFusedPlan* p, int k, int d, Arena& A) {
+  p->c_hi = A.take<float>((size_t)p->KP * p->DP, 1024);
+  p->c_lo = A.take<float>((size_t)p->KP * p->DP);
+  p->cnorm = A.take<float>(p->KP);
+  p->keytab = A.take<uint8_t>(512);
+  p->partials = A.take<float>((size_t)p->grid * k * d);
+  p->counts = A.take<int32_t>((size_t)p->grid * k);
+  p->cost_partials = A.take<double>(p->grid);
 }
 }  // namespace
 
@@ -994,10 +971,10 @@ bool b2k_fused_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const floa
   return b2k_fused_t_supported(ctx, n, d, k, X);   // large shapes: b2k_fused_t.cu (k <= 256, d <= 256)
 }
 
-int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, B2kFusedPlan* plan) {
+int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan) {
   Inst in;
   if (!pick_inst(d, k, &in) || ctx->force_variant_t) {
-    if (d % 4 == 0 && d <= 256 && k <= 256) return b2k_fused_t_plan(ctx, n, d, k, plan);
+    if (d % 4 == 0 && d <= 256 && k <= 256) return b2k_fused_t_plan(ctx, n, d, k, A, plan);
     return b2k_fail(ctx, B2K_ERR_UNSUPPORTED, "fused kernel: no instantiation for this (k, d)");
   }
   plan->variant = 0;
@@ -1019,57 +996,33 @@ int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, B2kFusedPlan* plan) {
   plan->grid = grid;
   plan->P = grid;
   plan->Pc = grid;
-  plan->scratch_bytes = plan_layout(*plan, k, d).total;
+  plan_layout(plan, k, d, A);
   return B2K_OK;
 }
 
-int b2k_fused_prepare(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d, int k,
+int b2k_fused_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
                       cudaStream_t s) {
-  if (plan.variant == 1) return b2k_fused_t_prepare(ctx, plan, plan_scratch, X, n, d, k, s);
+  if (plan.variant == 1) return b2k_fused_t_prepare(ctx, plan, X, n, d, norms, s);
   return B2K_OK;
 }
 
-int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, int64_t n, int k, int d,
-                            unsigned long long out[2], cudaStream_t s) {
+int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, unsigned long long out[2], cudaStream_t s) {
   out[0] = out[1] = 0ull;
   if (plan.variant != 1) return B2K_OK;
-  float* p;
-  int32_t* c;
-  double* cp;
-  unsigned long long* rs;
-  b2k_fused_t_views(plan, plan_scratch, n, k, d, &p, &c, &cp, &rs);
-  B2K_CUDA_OK(ctx, cudaMemcpyAsync(out, rs, 16, cudaMemcpyDeviceToHost, s));
+  B2K_CUDA_OK(ctx, cudaMemcpyAsync(out, plan.rstat, 16, cudaMemcpyDeviceToHost, s));
   B2K_CUDA_OK(ctx, cudaStreamSynchronize(s));
   return B2K_OK;
 }
 
-void b2k_fused_views(const B2kFusedPlan& plan, void* plan_scratch, int64_t n, int k, int d, float** partials,
-                     int32_t** counts, double** cost_partials) {
-  if (plan.variant == 1) {
-    b2k_fused_t_views(plan, plan_scratch, n, k, d, partials, counts, cost_partials, nullptr);
-    return;
-  }
-  PlanLayout L = plan_layout(plan, k, d);
-  char* b = static_cast<char*>(plan_scratch);
-  *partials = reinterpret_cast<float*>(b + L.off_partials);
-  *counts = reinterpret_cast<int32_t*>(b + L.off_counts);
-  *cost_partials = reinterpret_cast<double*>(b + L.off_cost);
-}
-
-int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d,
-                     const float* C, int k, int32_t* labels_out, float* mindist_out, bool do_update,
-                     const B2kLoopState* st, cudaStream_t s, const double* prev_counts) {
+int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int64_t n, int d, const float* C, int k,
+                     int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost, const B2kLoopState* st,
+                     cudaStream_t s, const double* prev_counts) {
   if (plan.variant == 1)
-    return b2k_launch_fused_t(ctx, plan, plan_scratch, X, n, d, C, k, labels_out, mindist_out, do_update,
-                              !do_update && (mindist_out != nullptr || ctx->want_cost), st, s, prev_counts);
-  PlanLayout L = plan_layout(plan, k, d);
-  char* b = static_cast<char*>(plan_scratch);
-  float* Chi = reinterpret_cast<float*>(b + L.off_chi);
-  float* Clo = reinterpret_cast<float*>(b + L.off_clo);
-  float* cnorm = reinterpret_cast<float*>(b + L.off_cnorm);
-
-  k_prep_centers_tc<<<(plan.KP * 32 + 255) / 256, 256, 0, s>>>(C, k, d, plan.KP, plan.DP, Chi, Clo, cnorm, st);
-  uint8_t* keytab = reinterpret_cast<uint8_t*>(b + L.off_tab);
+    return b2k_launch_fused_t(ctx, plan, X, n, d, C, k, labels_out, mindist_out, do_update,
+                              !do_update && (mindist_out != nullptr || need_cost), st, s, prev_counts);
+  uint8_t* keytab = plan.keytab;
+  k_prep_centers_tc<<<(plan.KP * 32 + 255) / 256, 256, 0, s>>>(C, k, d, plan.KP, plan.DP, plan.c_hi, plan.c_lo,
+                                                               plan.cnorm, st);
   k_balance_table<<<1, 128, 0, s>>>(do_update ? prev_counts : nullptr, k, plan.KP, keytab, keytab + 256, st);
   ctx->stats.kernel_launches += 2;
   B2K_CUDA_OK(ctx, cudaGetLastError());
@@ -1078,9 +1031,9 @@ int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch,
   B2K_TRY(encode_2d(ctx, &mx, X, (uint64_t)d, (uint64_t)n, (uint64_t)d * 4, CHUNK, TM,
                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
   const uint32_t cbox = (uint32_t)(plan.pair ? plan.KP / 2 : plan.KP);   // centre rows each CTA keeps in smem
-  B2K_TRY(encode_2d(ctx, &mh, Chi, (uint64_t)plan.DP, (uint64_t)plan.KP, (uint64_t)plan.DP * 4, CHUNK, cbox,
+  B2K_TRY(encode_2d(ctx, &mh, plan.c_hi, (uint64_t)plan.DP, (uint64_t)plan.KP, (uint64_t)plan.DP * 4, CHUNK, cbox,
                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
-  B2K_TRY(encode_2d(ctx, &ml, Clo, (uint64_t)plan.DP, (uint64_t)plan.KP, (uint64_t)plan.DP * 4, CHUNK, cbox,
+  B2K_TRY(encode_2d(ctx, &ml, plan.c_lo, (uint64_t)plan.DP, (uint64_t)plan.KP, (uint64_t)plan.DP * 4, CHUNK, cbox,
                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
 
   FusedArgs a{};
@@ -1088,12 +1041,12 @@ int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch,
   a.ntiles = (int)((n + TM - 1) / TM);
   a.k = k;
   a.d = d;
-  a.cnorm = cnorm;
+  a.cnorm = plan.cnorm;
   a.keytab = keytab;
   a.keyinv = keytab + 256;
-  a.partials = reinterpret_cast<float*>(b + L.off_partials);
-  a.counts = reinterpret_cast<int32_t*>(b + L.off_counts);
-  a.cost_partials = reinterpret_cast<double*>(b + L.off_cost);
+  a.partials = plan.partials;
+  a.counts = plan.counts;
+  a.cost_partials = plan.cost_partials;
   a.labels_out = labels_out;
   a.mind_out = mindist_out;
   a.do_update = do_update ? 1 : 0;

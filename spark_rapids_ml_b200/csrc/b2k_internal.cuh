@@ -45,21 +45,12 @@ struct b2k_ctx {
   int pair = 1;                  // option "pair": use the cta_group::2 instantiation where available (default on)
   int adaptive_path = 1;         // option "adaptive_path": a Lloyd loop on the large-shape kernel falls back to the generic
                                  // kernels for its remaining iterations when most rows need the exact fix-up
-  int lloyd_switched = 0;
-  int near_tie_hint = 0;         // set around the k-means|| candidate passes: prefer exact 128-centre chunks (d <= 128)        // the last lloyd_impl call did so (the fit's inertia pass follows it)
   int force_variant_t = 0;       // option "variant_t": route every supported shape through b2k_fused_t.cu (tests)
   int tma_box_rows = 0;          // option "tma_box_rows": rows per TMA box of b2k_debug_tma_stream (diagnostic; 0 = 128)
   int collect_recheck = 0;       // option "collect_recheck": fill stats.recheck_* (costs a stream sync per call)
-  int want_cost = 1;             // assign passes: compute the cost partial (set by assign_impl)
   int profile_fused = 0;         // record per-role blocked-cycle counters of the fused kernel
-  // Row norms of the large-shape kernel, shared by every pass of ONE b2k_kmeans_fit call (k-means|| candidate passes,
-  // the Lloyd loop, the inertia pass all see the same immutable X): computed by the first pass, reused by the rest.
-  const float* xnorm_scope_X = nullptr;   // non-null only inside b2k_kmeans_fit
-  int64_t xnorm_scope_n = 0;
-  int xnorm_scope_d = 0;
-  void* xnorm_cache = nullptr;            // float2 [xnorm_cache_rows]
+  void* xnorm_cache = nullptr;   // float2 [xnorm_cache_rows]: row norms shared by the passes of one fit (B2kNormScope)
   int64_t xnorm_cache_rows = 0;
-  int xnorm_cache_valid = 0;
   long long* prof_dev = nullptr;  // [grid][18 warps][8]
   int prof_grid = 0;
   // comm
@@ -105,6 +96,56 @@ int b2k_fail(b2k_ctx* ctx, int code, const std::string& msg);
 
 int b2k_scratch_reserve(b2k_ctx* ctx, size_t bytes);
 void b2k_copy_pool_destroy(b2k_ctx* ctx);
+
+// Bump allocator over device scratch.  A measuring arena (default-constructed: null base, unlimited capacity) only
+// counts bytes and hands out null pointers; a scratch user runs its layout on one to size b2k_scratch_reserve, then the
+// same layout on Arena(ctx->scratch, ctx->scratch_bytes) to carve its pointers.  A take past the capacity sets
+// `overflow`; the owner turns that into B2K_ERR_STATE before it launches anything.
+struct Arena {
+  char* base = nullptr;
+  size_t cap = SIZE_MAX;
+  size_t off = 0;
+  bool overflow = false;
+  Arena() = default;
+  Arena(void* b, size_t c) : base(static_cast<char*>(b)), cap(c) {}
+  template <typename T>
+  T* take(size_t count, size_t align = 256) {
+    off = (off + align - 1) / align * align;
+    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off += count * sizeof(T);
+    if (off > cap) overflow = true;
+    return p;
+  }
+};
+
+// Row norms of X shared by every large-shape pass of ONE b2k_kmeans_fit (the k-means|| candidate passes, the Lloyd loop
+// and the inertia pass all read the same immutable X): the first pass computes them into ctx->xnorm_cache, the rest
+// reuse them.  Owned by b2k_kmeans_fit; passes over any other matrix, and standalone lloyd / assign calls, get none.
+struct B2kNormScope {
+  const float* X;
+  int64_t n;
+  bool valid = false;   // ctx->xnorm_cache holds the norms of X
+};
+
+// Launches `kern` on clusters of two CTAs (the CTA pair of tcgen05 cta_group::2).
+template <typename... Params, typename... Args>
+int b2k_launch_pair(b2k_ctx* ctx, void (*kern)(Params...), int grid, int threads, size_t smem, cudaStream_t s,
+                    const Args&... args) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3((unsigned)grid);
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  B2K_CUDA_OK(ctx, cudaLaunchKernelEx(&cfg, kern, args...));
+  return B2K_OK;
+}
 
 // ------------------------------------------------------------------------------------------------
 // generic (any k, d) kernels — b2k_generic.cu
@@ -155,35 +196,48 @@ struct B2kFusedPlan {
   int variant = 0;           // 0: b2k_fused_tc.cu (k <= 128, d <= 128, 3xTF32); 1: b2k_fused_t.cu (k, d <= 256, 1xTF32 + recheck)
   int P = 0;                 // partial-sum slots the pass writes (variant 0: grid; variant 1: CTA pairs + 1 for the deferred rows)
   int Pc = 0;                // cost partials the pass writes (variant 0: grid; variant 1: grid + fix-up CTAs)
-  size_t scratch_bytes = 0;  // centre operands/cnorm + partials/counts/cost (+ row norms, variant 1)
+  // scratch carved by b2k_fused_plan (null when planned on a measuring arena)
+  float* partials = nullptr;         // [P][k*d] partial sums, [P][k] counts, [Pc] cost: b2k_launch_reduce_partials
+  int32_t* counts = nullptr;
+  double* cost_partials = nullptr;
+  float* cnorm = nullptr;            // variant 0: [KP] ||c||^2; variant 1: [512] {||c||^2, ||c - tf32(c)||}
+  uint8_t* keytab = nullptr;         // [2][256] cluster -> update slot table and its inverse
+  float* c_hi = nullptr;             // variant 0: tf32 split of the centres, [KP][DP] each
+  float* c_lo = nullptr;
+  float* ct = nullptr;               // variant 1: [256][DP] tf32-rounded centres
+  float* thr = nullptr;              // variant 1: [4] screening threshold coefficients
+  unsigned long long* rstat = nullptr;  // variant 1: {rows re-decided exactly, candidate distances evaluated}
+  float2* xnorm = nullptr;           // variant 1: [n] row norms (b2k_fused_prepare may point it at the fit's cache)
+  int2* fix_list = nullptr;          // variant 1: deferred rows, one segment of seg_cap entries per CTA pair
+  uint32_t* fix_masks = nullptr;     // variant 1: candidate masks for the first mask_cap entries of a segment
+  int32_t* fix_count = nullptr;      // variant 1: entries per segment
+  int seg_cap = 0, mask_cap = 0;
 };
 bool b2k_fused_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X);
-int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, B2kFusedPlan* plan);
-// Once per fit / lloyd / assign call, before the first b2k_launch_fused on this X (variant 1: row norms; variant 0: no-op)
-int b2k_fused_prepare(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d, int k,
+// Plans a fused pass over X[n, d] against k centres and carves its scratch from A.
+int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan);
+// Once per fit / lloyd / assign call, before the first b2k_launch_fused on this X (variant 1: row norms, into the plan's
+// scratch or, with a norm scope, into the fit's cache; variant 0: no-op)
+int b2k_fused_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
                       cudaStream_t s);
-// One fused pass: (labels_out, mindist_out optional) + partial sums/counts/cost into plan scratch.
+// One fused pass: (labels_out, mindist_out optional) + partial sums/counts/cost into the plan's scratch.
 // `do_update` = accumulate partial sums (Lloyd iteration) or labels only (assign/inertia pass).
-int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X,
-                     int64_t n, int d, const float* C, int k, int32_t* labels_out, float* mindist_out,
-                     bool do_update, const B2kLoopState* st, cudaStream_t s, const double* prev_counts = nullptr);
-// Views into the plan scratch after a fused pass (to feed b2k_launch_reduce_partials)
-void b2k_fused_views(const B2kFusedPlan& plan, void* plan_scratch, int64_t n, int k, int d, float** partials,
-                     int32_t** counts, double** cost_partials);
+// `need_cost`: the caller reads plan.cost_partials after an assign pass.  Variant 0 writes them on every assign pass
+// (and whenever mindist_out is given); variant 1 on an assign pass that asks for them or writes mindist_out.
+int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int64_t n, int d, const float* C, int k,
+                     int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost, const B2kLoopState* st,
+                     cudaStream_t s, const double* prev_counts = nullptr);
 // variant 1 diagnostics: {rows re-decided exactly, candidate distances evaluated} since the last b2k_fused_prepare
-int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, int64_t n, int k, int d,
-                            unsigned long long out[2], cudaStream_t s);
+int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, unsigned long long out[2], cudaStream_t s);
 
 // b2k_fused_t.cu (variant 1)
 bool b2k_fused_t_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X);
-int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, B2kFusedPlan* plan);
-void b2k_fused_t_views(const B2kFusedPlan& plan, void* plan_scratch, int64_t n, int k, int d, float** partials,
-                       int32_t** counts, double** cost_partials, unsigned long long** rstat);
-int b2k_fused_t_prepare(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d,
-                        int k, cudaStream_t s);
-int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, void* plan_scratch, const float* X, int64_t n, int d,
-                       const float* C, int k, int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost,
-                       const B2kLoopState* st, cudaStream_t s, const double* prev_counts);
+int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan);
+int b2k_fused_t_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
+                        cudaStream_t s);
+int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int64_t n, int d, const float* C, int k,
+                       int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost, const B2kLoopState* st,
+                       cudaStream_t s, const double* prev_counts);
 int b2k_launch_merge_chunk(b2k_ctx* ctx, float* md_acc, int32_t* lab_acc, const float* md, const int32_t* lab, int base,
                            int64_t n, const B2kLoopState* st, cudaStream_t s);
 int b2k_fused_encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,

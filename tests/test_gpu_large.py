@@ -194,6 +194,10 @@ def test_adaptive_path_leaves_the_screening_kernel_on_near_tie_data():
         assert res[1][0] == 8 and res[1][1] == 1
         assert res[0][0] == -1 and res[0][1] == 2 and res[0][2] > res[1][2] > 0
         c.set_option("adaptive_path", 1)
+        # a fit's inertia pass follows the path its Lloyd loop ended on: the generic kernels after the switch
+        out = c.kmeans_fit(_dev(Xd), k, init=Xd[:k].copy(), max_iter=iters, tol=-1.0)
+        st = c.stats()
+        assert st["path_switch_iter"] >= 0 and st["last_path"] == 1 and np.isfinite(out["inertia_"])
         Xb, ctr = ko.make_blobs(20000, d, k, seed=3)
         Cb = _dev((ctr + 0.25 * np.random.default_rng(0).normal(size=ctr.shape)).astype(np.float32))
         c.kmeans_lloyd(_dev(Xb), Cb, iters, -1.0)
