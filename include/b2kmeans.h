@@ -116,23 +116,14 @@ int b2k_ctx_create(int device, b2k_ctx** out);
 int b2k_ctx_destroy(b2k_ctx* ctx);
 /* Options: "kernel_path" (b2k_kernel_path), "time_kernels" (0/1/2: CUDA events around every fused launch; 2 = also
  * around the partial fold, the allreduce and finalize), "check_every" (iterations between host
- * convergence polls, default 4), "grid_limit" (cap on persistent CTAs, 0 = #SMs), "variant_t" (1 = route every shape with k, d <= 256 through the
+ * convergence polls, default 4), "variant_t" (1 = route every shape with k, d <= 256 through the
  * large-shape kernel b2k_fused_t.cu; default 0 = only shapes the 3xTF32 kernel does not cover), "collect_recheck"
  * (1 = lloyd/assign synchronise and fill b2k_stats.recheck_*), "adaptive_path" (see b2k_stats.path_switch_iter), "ingest_threads" (host threads of the pageable -> pinned
- * staging copy of b2k_ingest_append; 0 = default: 4, capped by half of the CPUs the process may use), "pair" (1 = use the
- * CTA-pair tcgen05 cta_group::2 kernel where instantiated, default 1); diagnostic builds only (`make trace` ->
- * libb2kmeans_trace.so, `-DB2K_PROBE=1`): "profile_fused" (0/1; the product build rejects it with
- * B2K_ERR_UNSUPPORTED at the next fused launch), "probe" (timing experiments that skip work). */
+ * staging copy of b2k_ingest_append; 0 = default: 4, capped by half of the CPUs the process may use).  Any other key
+ * fails with B2K_ERR_INVALID. */
 int b2k_ctx_set_option(b2k_ctx* ctx, const char* key, int64_t value);
 int b2k_get_stats(const b2k_ctx* ctx, b2k_stats* out);
-/* Diagnostics (diagnostic build + option "profile_fused"=1): per-CTA, per-warp-role cycle counters of the last fused
- * launch, layout [grid (+4 trace pseudo-CTAs)][warps][8] = {role cycles, 3 blocked-cycle counters, 2 stage timers, 0, 0}.
- * Synchronises the device. */
-int b2k_get_fused_profile(b2k_ctx* ctx, long long* out, int64_t cap, int* grid_out, int* warps_out);
 int b2k_reset_stats(b2k_ctx* ctx);
-/* Diagnostics: one pass of X[n, d] (d % 32 == 0) through an nslot x 16 KB TMA ring whose slots are released
- * `hold_cycles` after landing; *out_ms = device time.  Maps the bandwidth ceiling of the fused kernel's ring. */
-int b2k_debug_tma_stream(b2k_ctx* ctx, const float* X, int64_t n, int d, int nslot, int hold_cycles, float* out_ms);
 
 /* ---- communicator (NCCL over NVLink; one rank per process per GPU) ---- */
 int b2k_comm_unique_id(char out[B2K_UNIQUE_ID_BYTES]); /* rank 0 only */

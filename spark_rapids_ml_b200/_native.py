@@ -14,7 +14,7 @@ from typing import Any, Dict, Optional, Sequence, Tuple
 import numpy as np
 
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
-# B2K_LIB selects another build of the same library (e.g. the diagnostic libb2kmeans_trace.so from `make trace`)
+# B2K_LIB selects another build of the same library (e.g. one built from another revision)
 LIB_PATH = os.environ.get("B2K_LIB") or os.path.join(_PKG_DIR, "libb2kmeans.so")
 CSRC_DIR = os.path.join(_PKG_DIR, "csrc")
 
@@ -41,9 +41,7 @@ EXPORTED_SYMBOLS = (
     "b2k_ctx_destroy",
     "b2k_ctx_set_option",
     "b2k_get_stats",
-    "b2k_get_fused_profile",
     "b2k_reset_stats",
-    "b2k_debug_tma_stream",
     "b2k_comm_unique_id",
     "b2k_comm_init",
     "b2k_comm_destroy",
@@ -114,8 +112,6 @@ def load_library() -> ctypes.CDLL:
     L.b2k_ctx_set_option.argtypes = [vp, ctypes.c_char_p, i64]
     L.b2k_get_stats.argtypes = [vp, ctypes.POINTER(Stats)]
     L.b2k_reset_stats.argtypes = [vp]
-    L.b2k_get_fused_profile.argtypes = [vp, vp, i64, ctypes.POINTER(i32), ctypes.POINTER(i32)]
-    L.b2k_debug_tma_stream.argtypes = [vp, vp, i64, i32, i32, i32, ctypes.POINTER(ctypes.c_float)]
     L.b2k_comm_unique_id.argtypes = [ctypes.c_char_p]
     L.b2k_comm_init.argtypes = [vp, i32, i32, ctypes.c_char_p]
     L.b2k_comm_destroy.argtypes = [vp]
@@ -198,20 +194,6 @@ class Context:
         st = Stats()
         self._check(self._L.b2k_get_stats(self._h, ctypes.byref(st)))
         return {f: getattr(st, f) for f, _ in Stats._fields_}
-
-    def fused_profile(self) -> "np.ndarray":
-        """[grid, warps, 8] int64 cycle counters of the last fused launch (needs option profile_fused=1)."""
-        buf = np.zeros(1024 * 32 * 8, dtype=np.int64)
-        g, w = ctypes.c_int(0), ctypes.c_int(0)
-        self._check(self._L.b2k_get_fused_profile(self._h, buf.ctypes.data, buf.size, ctypes.byref(g), ctypes.byref(w)))
-        return buf[: g.value * w.value * 8].reshape(g.value, w.value, 8)
-
-    def debug_tma_stream(self, X: Any, nslot: int, hold_cycles: int = 0) -> float:
-        """ms for one TMA pass over X through an nslot x 16 KB ring (diagnostic)."""
-        ms = ctypes.c_float(0.0)
-        self._check(self._L.b2k_debug_tma_stream(self._h, X.data_ptr(), int(X.shape[0]), int(X.shape[1]), int(nslot),
-                                                 int(hold_cycles), ctypes.byref(ms)))
-        return float(ms.value)
 
     def reset_stats(self) -> None:
         self._check(self._L.b2k_reset_stats(self._h))

@@ -3,10 +3,7 @@
 // fixed-order partial reduce -> NCCL allreduce of one fused f64 buffer -> finalize, several iterations ahead
 // of the host; convergence lives on the device (B2kLoopState) and is polled every `check_every` iterations.
 #include <algorithm>
-#include <chrono>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <random>
 #include <vector>
@@ -73,7 +70,6 @@ extern "C" int b2k_ctx_destroy(b2k_ctx* ctx) {
   if (ctx->nccl) b2k_comm_destroy(ctx);
   b2k_copy_pool_destroy(ctx);
   if (ctx->scratch) cudaFree(ctx->scratch);
-  if (ctx->prof_dev) cudaFree(ctx->prof_dev);
   if (ctx->xnorm_cache) cudaFree(ctx->xnorm_cache);
   for (int i = 0; i < 2; ++i) {
     if (ctx->pinned[i]) cudaFreeHost(ctx->pinned[i]);
@@ -97,10 +93,6 @@ extern "C" int b2k_ctx_set_option(b2k_ctx* ctx, const char* key, int64_t value) 
   } else if (k == "check_every") {
     if (value < 1) return b2k_fail(ctx, B2K_ERR_INVALID, "check_every must be >= 1");
     ctx->check_every = (int)value;
-  } else if (k == "probe") {
-    ctx->probe = (int)value;
-  } else if (k == "pair") {
-    ctx->pair = value ? 1 : 0;
   } else if (k == "adaptive_path") {
     ctx->adaptive_path = value ? 1 : 0;
   } else if (k == "variant_t") {
@@ -109,15 +101,8 @@ extern "C" int b2k_ctx_set_option(b2k_ctx* ctx, const char* key, int64_t value) 
     if (value < 0 || value > 64) return b2k_fail(ctx, B2K_ERR_INVALID, "ingest_threads must be in [0, 64]");
     b2k_copy_pool_destroy(ctx);
     ctx->ingest_threads = (int)value;
-  } else if (k == "tma_box_rows") {
-    ctx->tma_box_rows = (int)value;
   } else if (k == "collect_recheck") {
     ctx->collect_recheck = value ? 1 : 0;
-  } else if (k == "profile_fused") {
-    ctx->profile_fused = value ? 1 : 0;
-  } else if (k == "grid_limit") {
-    if (value < 0) return b2k_fail(ctx, B2K_ERR_INVALID, "grid_limit must be >= 0");
-    ctx->grid_limit = (int)value;
   } else {
     return b2k_fail(ctx, B2K_ERR_INVALID, "unknown option: " + k);
   }
@@ -268,11 +253,6 @@ int chunked_assign_run(b2k_ctx* ctx, const ChunkedAssign& ca, const float* X, in
 static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, float* C, int max_iter, double tol,
                       B2kNormScope* norms, int* n_iter_out, double* shift_out, int* path_out, cudaStream_t s) {
   if (max_iter < 0) return b2k_fail(ctx, B2K_ERR_INVALID, "lloyd: max_iter < 0");
-  const bool dbg = std::getenv("B2K_DEBUG_TIMING") != nullptr;
-  const auto t_entry = std::chrono::steady_clock::now();
-  auto since = [&](std::chrono::steady_clock::time_point t0) {
-    return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  };
   const int path = ctx->kernel_path;
   // k > 256 (d <= 256): the assignment runs in 256-centre chunks on the large-shape kernel, the update stays generic
   const int chunk_ch = k > 256 ? chunked_assign_ch(ctx, path, false, n, d, k, X) : 0;
@@ -336,9 +316,6 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
   if (fused && max_iter > 0) B2K_TRY(b2k_fused_prepare(ctx, B.plan, X, n, d, norms, s));
   if (chunked && max_iter > 0) B2K_TRY(b2k_fused_prepare(ctx, ca.plan, X, n, d, norms, s));
   if (ctx->time_kernels) B2K_CUDA_OK(ctx, cudaEventRecord(loop0, s));
-  const double t_setup = since(t_entry);
-  const auto t_loop = std::chrono::steady_clock::now();
-  double t_first_burst = 0.0;
 
   // The host stays one burst ahead of the device: burst b + 1 is enqueued BEFORE the convergence flag of burst b is
   // read back, so a poll never drains the stream (every hot-loop kernel returns at once when `done` is set, which
@@ -382,7 +359,6 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
       if (e && nev_per_it == 5) B2K_CUDA_OK(ctx, cudaEventRecord(e[4], s));
       ++launched;
     }
-    if (t_first_burst == 0.0) t_first_burst = since(t_loop);
     burst_iters[slot] = fused_now ? burst : 0;
     B2K_CUDA_OK(ctx, cudaMemcpyAsync(&mirror[slot], B.st, sizeof(B2kLoopState), cudaMemcpyDeviceToHost, s));
     B2K_CUDA_OK(ctx, cudaEventRecord(poll_ev[slot], s));
@@ -410,9 +386,6 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
     slot ^= 1;
   }
   B2K_CUDA_OK(ctx, cudaStreamSynchronize(s));
-  if (dbg)
-    fprintf(stderr, "[b2k rank %d] lloyd host timing: setup %.3f ms, first burst enqueued after %.3f ms, loop %.3f ms (%d iterations)\n",
-            ctx->rank, t_setup, t_first_burst, since(t_loop), launched);
   if (have_pending && last_slot != 0) mirror[0] = mirror[last_slot];   // h_state[0] = the final state
   cudaEventDestroy(poll_ev[0]);
   cudaEventDestroy(poll_ev[1]);

@@ -36,27 +36,6 @@
 
 namespace {
 
-#ifndef B2K_MMA_WAIT
-#define B2K_MMA_WAIT mbar_wait_cluster
-#endif
-// -DB2K_PROBE=1 (make probe -> libb2kmeans_probe.so): option "probe" skips one stage's work (WRONG results; timing only):
-//   1 update rows   2 epilogue D processing   3 epilogue exchange   4 MMAs   5 sort   6 remote rows read locally
-#ifndef B2K_PROBE
-#define B2K_PROBE 0
-#endif
-#if B2K_PROBE
-#define B2K_PROBE_IS(x) (args.probe == (x))
-// event trace (option "profile_fused"): clock64 of 16 events x 8 steps (20..27) of CTAs 0 and 1, read back through
-// b2k_get_fused_profile: [cta][step][event]
-#define B2K_TR(itv, ev)                                                                                   \
-  do {                                                                                                    \
-    if (args.trace != nullptr && blockIdx.x < 2 && (itv) >= 20 && (itv) < 28 && (threadIdx.x & 31) == 0) \
-      args.trace[((int)blockIdx.x * 8 + ((itv)-20)) * 16 + (ev)] = clock64();                             \
-  } while (0)
-#else
-#define B2K_PROBE_IS(x) false
-#define B2K_TR(itv, ev) ((void)0)
-#endif
 #include "b2k_ptx.cuh"
 
 constexpr int TN = 128;                      // X rows per step = UMMA N (64 per CTA of the pair)
@@ -312,8 +291,6 @@ struct TArgs {
   int32_t* labels_out;     // [n] or NULL
   float* mind_out;         // [n] or NULL
   int need_cost;
-  int probe;
-  long long* trace;
   unsigned long long* rstat;   // [2] deferred (rechecked) rows, candidates evaluated (diagnostics) or NULL
   // deferred rows: CTA pair p appends to fix_list[p * seg_cap ..] in step order (a fixed function of the data) and
   // writes fix_count[p] when it is done; entries below mask_cap also carry their 256-bit candidate mask
@@ -441,7 +418,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
       // The update warps run decoupled (no per-step barrier among them): rows per warp and step are Poisson(4), and a
       // barrier would make every step wait for its most loaded warp (measured: 5-7 k cycles per step against 2.5 k mean).
       mbar_wait_nocall(bar(B_LFULL + b), bph);
-      if (u == 0) B2K_TR(it, 11);
       // The x_full phases of this step completed before the MMA consumed the slots, which happens-before the
       // commit, the epilogue and hence lab_full: the rows are in shared memory (both CTAs).
       const uint32_t slot0 = ring + (uint32_t)((ss * NCH + (lane >> 3)) * SLOT_BYTES);
@@ -460,7 +436,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
         auto load_row = [&](int colr, uint64_t (&v)[UPL][2]) {
           const int lrow = colr & 63;
           const uint32_t a0 = slot0 + (((uint32_t)(lrow * 128 + ((lrow & 7) << 4))) ^ unit_js);
-          if ((uint32_t)(colr >> 6) == rank || B2K_PROBE_IS(6)) {
+          if ((uint32_t)(colr >> 6) == rank) {
 #pragma unroll
             for (int i = 0; i < UPL; ++i) lds128_2(a0 + (uint32_t)(i * 4 * SLOT_BYTES), v[i][0], v[i][1]);
           } else {
@@ -487,13 +463,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
         // two rows in flight: the load of row i + 1 is issued before row i is added (its latency — 30 cycles local,
         // several hundred through DSMEM under load — is the cost of a row; measured ~700-1000 cycles per row serial)
         uint64_t vA[UPL][2], vB[UPL][2];
-        if (u == 0) B2K_TR(it, 1);
         int pend = 0, cP = 0;   // pend: 0 nothing in flight, 1 = vA, 2 = vB (the buffers alternate: no register copies)
 #pragma unroll 1
         for (int sx = 0; sx < 4; ++sx) {
           uint32_t m = __ballot_sync(0xffffffffu, ((vmask >> sx) & 1u) != 0u &&
                                                        (((keyp >> (8 * sx)) & 255u) - (uint32_t)k0) < (uint32_t)CPW);
-          if (B2K_PROBE_IS(1) || B2K_PROBE_IS(9)) m = 0u;
           while (m) {
             const int bit = __ffs(m) - 1;
             m &= m - 1;
@@ -547,7 +521,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
         }
       }
       __syncwarp();
-      if (u == 0) B2K_TR(it, 12);
       if (lane == 0) {
         // the rows were consumed (their values fed the adds above) before these arrivals: relaxed is enough for the
         // write-after-read hand-back of the slots to the TMA producers of both CTAs
@@ -593,7 +566,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
       // (measured: 8 of them per step put 3.6 k cycles on the MMA issuer).  What these barriers order is async-proxy
       // traffic (TMA writes / UMMA reads) and TMEM (tcgen05 fences), not generic-proxy data in the peer's memory.
       mbar_wait_nocall(bar(B_SFREE + ss), sph ^ 1u);
-      B2K_TR(it, 0);
 #pragma unroll 1
       for (int c = 0; c < NCH; ++c) {
         const int slot = ss * NCH + c;
@@ -616,47 +588,24 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
       const uint32_t sph = (uint32_t)(it / NSTEP) & 1u;
       mbar_wait_nocall(bar(B_DEMPTY + b), bph ^ 1u);
       tc_fence_after();
-      B2K_TR(it, 2);
       const uint32_t d_tmem = tmem_base + D_OFF + b * TN;
-#if B2K_PROBE
-      if (B2K_PROBE_IS(12)) {   // all MMAs of the step back to back, no waits (timing only)
-        if (elect_one()) {
-#pragma unroll 1
-          for (int c = 0; c < NCH; ++c) {
-            const uint32_t bx = ring + (ss * NCH + c) * SLOT_BYTES;
-#pragma unroll
-            for (int ks = 0; ks < CHUNK / 8; ++ks)
-              tc_mma_ts_tf32_pair(d_tmem, tmem_base + (uint32_t)(c * CHUNK + ks * 8), make_kmajor_sw128_desc(bx + ks * 32),
-                                  idesc, (c | ks) != 0 ? 1u : 0u);
-          }
-          tc_commit_pair(bar(B_DFULL + b));
-        }
-        __syncwarp();
-        B2K_TR(it, 4);
-        continue;
-      }
-#endif
 #pragma unroll 1
       for (int c = 0; c < NCH; ++c) {
         const int slot = ss * NCH + c;
-        if ((c % XG) == 0 && !B2K_PROBE_IS(10)) {
+        if ((c % XG) == 0) {
           mbar_wait_nocall(bar(B_XFULL + slot / XG), sph);
           tc_fence_after();
         }
-        if (c == 0) B2K_TR(it, 3);
-        if (c == NCH - 1) B2K_TR(it, 14);
         if (elect_one()) {
           const uint32_t bx = ring + slot * SLOT_BYTES;
 #pragma unroll
           for (int ks = 0; ks < CHUNK / 8; ++ks)
-            if ((!B2K_PROBE_IS(4) || (c | ks) == 0) && (!B2K_PROBE_IS(7) || ks == 0) && (!B2K_PROBE_IS(8) || ks < 2))
-              tc_mma_ts_tf32_pair(d_tmem, tmem_base + (uint32_t)(c * CHUNK + ks * 8), make_kmajor_sw128_desc(bx + ks * 32),
+            tc_mma_ts_tf32_pair(d_tmem, tmem_base + (uint32_t)(c * CHUNK + ks * 8), make_kmajor_sw128_desc(bx + ks * 32),
                                 idesc, (c | ks) != 0 ? 1u : 0u);
           if (c == NCH - 1) tc_commit_pair(bar(B_DFULL + b));
         }
         __syncwarp();
       }
-      B2K_TR(it, 4);
     }
    }
   } else if (warp < W_UPD0) {
@@ -702,16 +651,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
       // per-row key offset ||x||^2 + thr: dist' + offset = ||x - c||^2 + thr +- E > 0, so that the float bits of a key
       // order like unsigned integers, with the key's resolution relative to the true squared distance
       xoff_s[col] = fmaf(xn, xn, thr);
-      if (threadIdx.x == 0 && !B2K_PROBE_IS(9)) mbar_expect_tx(bar(B_PX + b), PX_BYTES);   // the peer's partials of this step
+      if (threadIdx.x == 0) mbar_expect_tx(bar(B_PX + b), PX_BYTES);   // the peer's partials of this step
       // two barriers, two warps: even a completed wait costs several hundred cycles, so they are polled in parallel and
       // joined by the hardware barrier below
       if (w == 0) mbar_wait(bar(B_DFULL + b), bph);
       if (w == 1) mbar_wait(bar(B_LEMPTY + b), bph ^ 1u);   // lab[b] of step it - 2 has been consumed by the update role
       asm volatile("bar.sync 1, 128;" ::: "memory");
       tc_fence_after();
-      if (w == 0) B2K_TR(it, 5);
 #pragma unroll 1
-      for (int g = 0; g < (B2K_PROBE_IS(9) ? 0 : TN / 32); ++g) {
+      for (int g = 0; g < TN / 32; ++g) {
         uint32_t v[2][16];
         const uint32_t ta = tmem_base + ((uint32_t)(w * 32) << 16) + (uint32_t)(D_OFF + b * TN + g * 32);
         tmem_ld_16x256b_x4(ta, v[0]);
@@ -743,15 +691,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
         st_async_v2(part_peer0 + (uint32_t)pi * 8u, m1[0], m2[0], px_peer0 + 8u * (uint32_t)b);
       }
       tc_fence_before();
-      if (w == 0) B2K_TR(it, 6);
       asm volatile("bar.sync 1, 128;" ::: "memory");   // this CTA's partials
       // D of this parity is drained in this CTA (nothing below reads TMEM)
       if (threadIdx.x == 0) {
         asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(dempty_leader + 8u * (uint32_t)b)
                      : "memory");
       }
-      if (!B2K_PROBE_IS(9)) mbar_wait(bar(B_PX + b), bph);                    // the peer's partials
-      if (w == 0) B2K_TR(it, 7);
+      mbar_wait(bar(B_PX + b), bph);                    // the peer's partials
       // combine the 8 partials of my column (source s8 = the 32 clusters [32 s8, 32 s8 + 32))
       uint32_t M1 = 0xffffffffu, M2 = 0xffffffffu;
       uint2 pp[8];
@@ -761,10 +707,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
         merge2(M1, M2, pp[s8].x, pp[s8].y);
       }
       int label = (int)(M1 & 255u);
-      if (B2K_PROBE_IS(9)) label = (col * 2 + (int)rank) & 255;
       const float M1f = __uint_as_float(M1 & 0xffffff00u);
-      const bool flag = valid && ((__uint_as_float(M2 & 0xffffff00u) - M1f) < thr) &&
-                        !(B2K_PROBE_IS(4) || B2K_PROBE_IS(7) || B2K_PROBE_IS(8) || B2K_PROBE_IS(9) || B2K_PROBE_IS(10) || B2K_PROBE_IS(11) || B2K_PROBE_IS(12));
+      const bool flag = valid && ((__uint_as_float(M2 & 0xffffff00u) - M1f) < thr);
       const uint32_t fl = __ballot_sync(0xffffffffu, flag);
       if (lane == 0) flagw_s[w] = fl;
       asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -772,7 +716,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
 #pragma unroll
       for (int i = 0; i < 4; ++i) fw[i] = flagw_s[i];
       const int nflag = __popc(fw[0]) + __popc(fw[1]) + __popc(fw[2]) + __popc(fw[3]);
-      if (w == 0) B2K_TR(it, 8);
       if (nflag != 0) {
         // ---- deferred rows (identical flags in both CTAs): entry seg_cnt + (rank of the column among the step's flagged
         // columns), written by the row's owner.  Candidates = every cluster whose approximate distance may be within thr of
@@ -801,7 +744,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
           ++n_flag;
         }
         seg_cnt += nflag;
-        if (w == 0) B2K_TR(it, 9);
       }
       if (flag) label = -1;
       // ---- publish the labels: the update warps find their rows themselves (invalid and deferred rows: -1) ----
@@ -809,7 +751,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused_t(const __grid_constant__
       if (valid && label >= 0 && (uint32_t)(col >> 6) == rank && args.labels_out != nullptr) args.labels_out[grow] = label;
       asm volatile("bar.sync 1, 128;" ::: "memory");
       if (threadIdx.x == 0) mbar_arrive(bar(B_LFULL + b));
-      if (w == 0) B2K_TR(it, 10);
     }
     if (threadIdx.x == 0 && rank == 0) args.fix_count[pairid] = seg_cnt;
     if (args.rstat != nullptr) {
@@ -1105,7 +1046,6 @@ int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPl
   plan->pair = 1;
   const int64_t nsteps = (n + TN - 1) / TN;
   int grid = ctx->sm_count & ~1;
-  if (ctx->grid_limit > 0 && ctx->grid_limit < grid) grid = ctx->grid_limit & ~1;
   if (nsteps * 2 < grid) grid = (int)nsteps * 2;
   if (grid < 2) grid = 2;
   plan->grid = grid;
@@ -1174,16 +1114,6 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, i
   a.labels_out = labels_out;
   a.mind_out = mindist_out;
   a.need_cost = need_cost ? 1 : 0;
-  a.probe = ctx->probe;
-  a.trace = nullptr;
-#if B2K_PROBE
-  if (ctx->profile_fused) {
-    if (!ctx->prof_dev) B2K_CUDA_OK(ctx, cudaMalloc(&ctx->prof_dev, (size_t)1024 * 26 * 8 * sizeof(long long)));
-    B2K_CUDA_OK(ctx, cudaMemsetAsync(ctx->prof_dev, 0, 2 * 26 * 8 * sizeof(long long), s));
-    a.trace = ctx->prof_dev;
-    ctx->prof_grid = 2;
-  }
-#endif
   a.rstat = plan.rstat;
   a.fix_list = plan.fix_list;
   a.fix_masks = plan.fix_masks;

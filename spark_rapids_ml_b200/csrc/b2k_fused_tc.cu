@@ -34,36 +34,6 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // configuration
 // ------------------------------------------------------------------------------------------------
-// Diagnostic build (make trace -> libb2kmeans_trace.so): per-stage cycle counters and a per-tile event trace on top of
-// the blocked-cycle counters of option "profile_fused".  Off in the product build: even the predicated-off timer
-// reads cost ~10 % of the kernel's speed (register pressure in the convert / epilogue loops; measured).
-// -DB2K_PROBE=1: timing experiments selected by option "probe" (they skip work: WRONG results; never in the product)
-#ifndef B2K_PROBE
-#define B2K_PROBE 0
-#endif
-#ifndef B2K_MMA_WAIT
-#define B2K_MMA_WAIT mbar_wait   // CTA scope: a cluster-scope acquire appends CCTL.IVALL (L1 invalidate) to every wait (r02)
-#endif
-#ifndef B2K_TRACE
-#define B2K_TRACE 0
-#endif
-#if B2K_TRACE
-#define B2K_T0(v) const long long v = prof ? clock64() : 0
-#define B2K_TACC(slot, expr) do { if (prof) pw[slot] += (expr); } while (0)
-#define B2K_TR(ti, ev) tr(ti, ev)
-#define B2K_TRACE_CTAS 4
-#else
-#define B2K_T0(v) ((void)0)
-#define B2K_TACC(slot, expr) ((void)0)
-#define B2K_TR(ti, ev) ((void)0)
-#define B2K_TRACE_CTAS 0
-#endif
-#ifndef B2K_PACKED_SPLIT
-#define B2K_PACKED_SPLIT 1
-#endif
-#ifndef B2K_NSLOT_CAP
-#define B2K_NSLOT_CAP 13
-#endif
 constexpr int TM = 128;            // rows per tile (UMMA M)
 constexpr int CHUNK = 32;          // f32 per 128-byte swizzle row = one TMA box / K chunk
 constexpr int SLOT_BYTES = TM * CHUNK * 4;  // 16 KB
@@ -116,7 +86,7 @@ struct Cfg {
   // static shared memory), so there is no alignment slack.
   static constexpr int MISC = 1024 /*xnorm*/ + KP * 4 + BAR_BYTES + 64 + SL::BYTES;
   static constexpr int NSLOT_RAW = (int)((SMEM_LIMIT - 2 * C_BYTES - MISC) / SLOT_BYTES);
-  static constexpr int NSLOT = NSLOT_RAW > B2K_NSLOT_CAP ? B2K_NSLOT_CAP : NSLOT_RAW;
+  static constexpr int NSLOT = NSLOT_RAW > 13 ? 13 : NSLOT_RAW;   // ring depth capped at 13 slots
   static_assert(NSLOT >= NCH + 1, "ring too small");
   static constexpr int OFF_RING = 0;
   static constexpr int OFF_CHI = NSLOT * SLOT_BYTES;
@@ -226,10 +196,8 @@ struct FusedArgs {
   int32_t* labels_out;     // [n] or NULL
   float* mind_out;         // [n] or NULL
   int do_update;
-  int probe;               // -DB2K_PROBE=1 builds: timing experiment selector (skips work; wrong results)
   int need_cost;           // compute ||x||^2, min distance and the cost partial (assign / inertia passes)
   const B2kLoopState* st;
-  long long* prof;         // [grid][NWARPS][8] cycle counters or NULL
 };
 
 // NC: the pass also produces ||x||^2, the min distance and the cost partial (assign / inertia passes); a template
@@ -260,21 +228,7 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-#if B2K_TRACE
-  const bool prof = args.prof != nullptr;
-#else
-  constexpr bool prof = false;   // the cycle counters exist in the diagnostic build only (they cost speed: code size)
-#endif
   constexpr bool need_cost = NC;
-  long long pw[6] = {0, 0, 0, 0, 0, 0};   // blocked cycles per barrier kind (role specific)
-  const long long t_role0 = prof ? clock64() : 0;
-#if B2K_TRACE
-  // event trace of 16 consecutive tiles (200..215) for CTAs 0 and 1, stored behind the per-warp counters
-  long long* trace = (prof && blockIdx.x < 2) ? args.prof + (size_t)gridDim.x * NWARPS * 8 + blockIdx.x * 256 : nullptr;
-  auto tr = [&](int ti, int ev) {
-    if (trace != nullptr && ti >= 200 && ti < 216 && (threadIdx.x & 31) == 0) trace[(ti - 200) * 16 + ev] = clock64();
-  };
-#endif
 
   // ---- one-time setup ----
   if (warp == W_TMA && lane == 0) {
@@ -352,14 +306,12 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
       const int tile = tile_of(ti);
 #pragma unroll 1
       for (int c = 0; c < G::NCH; ++c) {
-        mbar_wait_p(bar(G::B_XEMPTY + xs), xph ^ 1u, prof, pw[0]);
+        mbar_wait(bar(G::B_XEMPTY + xs), xph ^ 1u);
         if (elect_one()) {
           mbar_expect_tx(bar(G::B_XFULL + xs), SLOT_BYTES);
           tma_load_2d(ring + xs * SLOT_BYTES, &mapX, bar(G::B_XFULL + xs), c * CHUNK, tile * TM);
         }
         __syncwarp();
-        if (c == 0) B2K_TR(ti, 0);
-        if (c == G::NCH - 1) B2K_TR(ti, 1);
         if (++xs == G::NSLOT) { xs = 0; xph ^= 1u; }
       }
     }
@@ -372,21 +324,15 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
     for (int ti = 0; ti < ((PAIR && rank != 0) ? 0 : nit); ++ti) {   // PAIR: only the leader CTA issues
       const int b = ti & 1;
       const uint32_t bph = (uint32_t)(ti >> 1) & 1u;
-      if constexpr (PAIR) B2K_MMA_WAIT(bar(G::B_DEMPTY + b), bph ^ 1u);
-      else mbar_wait_p(bar(G::B_DEMPTY + b), bph ^ 1u, prof, pw[0]);
+      // CTA-scope waits, PAIR included: a cluster-scope acquire makes ptxas append CCTL.IVALL (L1 invalidate) to every
+      // wait, and what these barriers order is TMEM traffic (tcgen05 fences on both sides)
+      mbar_wait(bar(G::B_DEMPTY + b), bph ^ 1u);
       tc_fence_after();
-      B2K_TR(ti, 13);
       const uint32_t d_tmem = tmem_base + D_OFF + b * KP;
 #pragma unroll 1
       for (int c = 0; c < G::NCH; ++c) {
-        {
-          if constexpr (PAIR) B2K_MMA_WAIT(bar(G::B_AFULL + as), aph);
-          else mbar_wait_p(bar(G::B_AFULL + as), aph, prof, pw[1]);
-        }
+        mbar_wait(bar(G::B_AFULL + as), aph);
         tc_fence_after();
-        if (c == 0) B2K_TR(ti, 14);
-        if (c == G::NCH - 2) B2K_TR(ti, 10);
-        if (c == G::NCH - 1) B2K_TR(ti, 11);
         if (elect_one()) {
           const uint32_t a_hi = tmem_base + as * A_COLS;
           const uint32_t a_lo = a_hi + CHUNK;
@@ -397,14 +343,6 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
             const uint64_t dhi = make_kmajor_sw128_desc(bhi + ks * 32);
             const uint64_t dlo = make_kmajor_sw128_desc(blo + ks * 32);
             if constexpr (PAIR) {
-#if B2K_PROBE   // probe 4 / 5: only 1 / 2 of the 3 products
-              if (args.probe == 4) { tc_mma_ts_tf32_pair(d_tmem, a_hi + ks * 8, dhi, idesc, (c | ks) != 0 ? 1u : 0u); continue; }
-              if (args.probe == 5) {
-                tc_mma_ts_tf32_pair(d_tmem, a_lo + ks * 8, dhi, idesc, (c | ks) != 0 ? 1u : 0u);
-                tc_mma_ts_tf32_pair(d_tmem, a_hi + ks * 8, dhi, idesc, 1u);
-                continue;
-              }
-#endif
               tc_mma_ts_tf32_pair(d_tmem, a_lo + ks * 8, dhi, idesc, (c | ks) != 0 ? 1u : 0u);
               tc_mma_ts_tf32_pair(d_tmem, a_hi + ks * 8, dlo, idesc, 1u);
               tc_mma_ts_tf32_pair(d_tmem, a_hi + ks * 8, dhi, idesc, 1u);
@@ -423,7 +361,6 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
           }
         }
         __syncwarp();
-        if (c == G::NCH - 1) B2K_TR(ti, 12);
         if (++as == NA) { as = 0; aph ^= 1u; }
       }
     }
@@ -434,7 +371,6 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
     const uint32_t lane_field = (uint32_t)(q * 32) << 16;
     const uint32_t swz = (uint32_t)(r & 7);
     const uint64_t kSplitA = pack2(8193.f, 8193.f), kSplitB = pack2(-8192.f, -8192.f);
-    (void)kSplitA; (void)kSplitB;
     int xs = 0, as = 0;
     uint32_t xph = 0, aph = 0;
     // PAIR: this CTA's centre half must have landed before its first a_full signal reaches the leader
@@ -465,14 +401,12 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
           const int p = warp - W_CONVERT0;
           if (p < 2 * CG) {
             const int g = p >> 1;
-            if ((p & 1) == 0) mbar_wait_p(bar(G::B_XFULL + (g == 0 ? xs_g[0] : xs_g[CG - 1])), g == 0 ? xp_g[0] : xp_g[CG - 1], prof, pw[0]);
-            else mbar_wait_p(bar(G::B_AEMPTY + (g == 0 ? as_g[0] : as_g[CG - 1])), g == 0 ? ap_g[0] : ap_g[CG - 1], prof, pw[1]);
+            if ((p & 1) == 0) mbar_wait(bar(G::B_XFULL + (g == 0 ? xs_g[0] : xs_g[CG - 1])), g == 0 ? xp_g[0] : xp_g[CG - 1]);
+            else mbar_wait(bar(G::B_AEMPTY + (g == 0 ? as_g[0] : as_g[CG - 1])), g == 0 ? ap_g[0] : ap_g[CG - 1]);
           }
         }
         asm volatile("bar.sync 6, 128;" ::: "memory");
         tc_fence_after();
-        B2K_T0(t_c0);
-        if (warp == W_CONVERT0) { if (c == 0) B2K_TR(ti, 9); if (c + CG >= G::NCH) B2K_TR(ti, 2); }
         // need_cost is hoisted out of the element loop (two copies of the body): a per-float4 branch costs as
         // much issue bandwidth as a fifth of the split itself
         auto convert_group = [&](auto) {
@@ -490,11 +424,10 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
               const int j = h * 4 + j2;
               float4 v = lds128(rowaddr + (((uint32_t)j ^ swz) << 4));
               float e[4] = {v.x, v.y, v.z, v.w};
-#if B2K_PACKED_SPLIT
               // Veltkamp split with packed fp32 pairs: t = fl(8193 x); hi = t - 8192 x (one FFMA2, exact) is x rounded
               // to nearest at 11 significant bits = a tf32 value (the tensor core's truncation is then a no-op);
               // l = x - hi is exact.  lo = RN_tf32(l) through the +1/2 ulp word trick (hardware truncates).
-              // 2.5 issue slots per element instead of 4.
+              // 2.5 issue slots per element instead of 4 for the unpacked form.
 #pragma unroll
               for (int t = 0; t < 4; t += 2) {
                 const uint64_t x2 = pack2(e[t], e[t + 1]);
@@ -510,38 +443,16 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
                 lo[j2 * 4 + t + 1] = __float_as_uint(l1) + 0x1000u;
                 if constexpr (NC) xn = fmaf(e[t + 1], e[t + 1], fmaf(e[t], e[t], xn));
               }
-#else
-#pragma unroll
-              for (int t = 0; t < 4; ++t) {
-                // The tensor core TRUNCATES fp32 operands to tf32 (measured: tools/probe_trunc.py).  Adding half a
-                // tf32 ulp to the stored word turns that truncation into round-to-nearest, for hi and for lo:
-                //   hi = RN_tf32(x)  (|x - hi| <= 2^-12 |x|),  lo = RN_tf32(x - hi)  (x - hi is exact in fp32)
-                // so x.c = hi.c_hi + lo.c_hi + hi.c_lo + O(2^-23 |x||c|): fp32-class accuracy from three tf32 MMAs.
-                // (Storing hi un-rounded saves one ALU op per element but doubles the residual; a golden-fixture row
-                // with a 3e-7 relative margin then flips, so the rounding stays.)
-                const uint32_t hs = __float_as_uint(e[t]) + 0x1000u;
-                const float l = e[t] - __uint_as_float(hs & 0xffffe000u);   // exact
-                hi[j2 * 4 + t] = hs;
-                lo[j2 * 4 + t] = __float_as_uint(l) + 0x1000u;
-                if constexpr (NC) xn = fmaf(e[t], e[t], xn);
-              }
-#endif
             }
             tmem_st_x16(a_addr + h * 16, hi);
             tmem_st_x16(a_addr + CHUNK + h * 16, lo);
           }
         }
         };
-#if B2K_PROBE
-        if (args.probe == 9) { /* skip */ } else
-#endif
         convert_group(std::integral_constant<bool, NC>{});
         tmem_wait_st();
         tc_fence_before();
-        asm volatile("bar.sync 3, 128;" ::: "memory");
-        B2K_T0(t_c1);
-        if (warp == W_CONVERT0 && c + CG >= G::NCH) B2K_TR(ti, 3);
-        B2K_TACC(3, t_c1 - t_c0);                  // whole group: loads + split + st + wait + barrier   // the 4 convert warps (hardware barrier: no polling)
+        asm volatile("bar.sync 3, 128;" ::: "memory");   // the 4 convert warps (hardware barrier: no polling)
         if (warp == W_CONVERT0 && lane == 0) {            // one arrival per role keeps the waiters' wake-ups low
 #pragma unroll
           for (int g = 0; g < CG; ++g) {
@@ -550,10 +461,9 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
             mbar_arrive(bar(G::B_XEMPTY + xs_g[g]));
           }
         }
-        B2K_TACC(4, clock64() - t_c1);              // signalling (leader: remote + local arrives)
       }
       if (need_cost) {
-        mbar_wait_p(bar(G::B_NEMPTY + b), bph ^ 1u, prof, pw[2]);
+        mbar_wait(bar(G::B_NEMPTY + b), bph ^ 1u);
         xnorm_s[b * TM + r] = xn;
         __syncwarp();
         if (lane == 0) mbar_arrive(bar(G::B_NFULL + b));
@@ -569,17 +479,11 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
       const int tile = tile_of(ti);
       const int b = ti & 1;
       const uint32_t bph = (uint32_t)(ti >> 1) & 1u;
-      if (warp == W_EPI0) mbar_wait_p(bar(G::B_DFULL + b), bph, prof, pw[0]);
+      if (warp == W_EPI0) mbar_wait(bar(G::B_DFULL + b), bph);
       asm volatile("bar.sync 5, 128;" ::: "memory");
       tc_fence_after();
-      B2K_T0(t_e0);
-      if (warp == W_EPI0) B2K_TR(ti, 4);
       float best = __int_as_float(0x7f800000);
       int bj = 0;
-#if B2K_PROBE
-      if (args.probe == 8) { bj = r & (KP - 1); best = 0.f; } else
-#endif
-      {
       // argmin over j in index order with strict '<' (lowest index wins ties).  Four independent chains of 8
       // consecutive candidates, merged in ascending order, give the same winner with a 12-deep instead of a
       // 32-deep dependent compare/select chain per 32 columns.
@@ -640,11 +544,7 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
         for (int q4 = 0; q4 < 2; ++q4)
           if (cb[q4] < best) { best = cb[q4]; bj = ci[q4]; }
       }
-      }
       tc_fence_before();
-      B2K_T0(t_e1);
-      if (warp == W_EPI0) B2K_TR(ti, 5);
-      B2K_TACC(3, t_e1 - t_e0);                    // TMEM load + argmin
 
       const int64_t grow = (int64_t)tile * TM + r;
       const bool valid = grow < args.n;
@@ -694,7 +594,7 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
         for (int q2 = 0; q2 < 3; ++q2)
           if (q2 < q) pos += (int)cnt[q2 * KP + key];
       }
-      mbar_wait_p(bar(G::B_LEMPTY + b), bph ^ 1u, prof, pw[2]);
+      mbar_wait(bar(G::B_LEMPTY + b), bph ^ 1u);
       if (valid) rows_sorted[pos] = (uint16_t)(r * 128 + ((r & 7) << 4));
       if (q == 0) {
 #pragma unroll
@@ -706,12 +606,10 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
       }
       asm volatile("bar.sync 4, 128;" ::: "memory");      // row list complete
       if (warp == W_EPI0 && lane == 0) mbar_arrive(bar(G::B_LFULL + b));
-      if (warp == W_EPI0) B2K_TR(ti, 6);
-      B2K_TACC(4, clock64() - t_e1);               // sort (includes the lab_empty wait counted in pw[2])
       // off the critical path: outputs and cost
       if (valid && args.labels_out) args.labels_out[grow] = bj;
       if (need_cost) {
-        mbar_wait_p(bar(G::B_NFULL + b), bph, prof, pw[1]);
+        mbar_wait(bar(G::B_NFULL + b), bph);
         const float xn = xnorm_s[b * TM + r];
         const float md = fmaxf(xn + best, 0.f);
         if (valid) {
@@ -751,13 +649,11 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
       const int b = ti & 1;
       const uint32_t bph = (uint32_t)(ti >> 1) & 1u;
       // one warp polls the mbarrier, the other 15 park in a hardware barrier (no issue slots, no wake-ups)
-      if (warp == W_UPD0) mbar_wait_p(bar(G::B_LFULL + b), bph, prof, pw[0]);
+      if (warp == W_UPD0) mbar_wait(bar(G::B_LFULL + b), bph);
       asm volatile("bar.sync 7, 512;" ::: "memory");
       // The x_full phases of this tile's slots completed before the convert warps consumed them, which
       // happens-before the MMA commit, the epilogue and hence this tile's lab_full: no need to poll them again.
-      B2K_T0(t_w0);
-      if (warp == W_UPD0) B2K_TR(ti, 7);
-      if (args.do_update && !(B2K_PROBE && args.probe == 6)) {
+      if (args.do_update) {
         const uint16_t* rows_sorted = reinterpret_cast<const uint16_t*>(sort_s + SL::ROWS) + b * 128;
         const uint8_t* start = sort_s + SL::START + b * SL::SP;
         uint32_t unit_base[G::UPL];
@@ -805,11 +701,7 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
           }
         }
       }
-      B2K_T0(t_w1);
-      B2K_TACC(3, t_w1 - t_w0);                    // this warp's rows
       asm volatile("bar.sync 2, 512;" ::: "memory");     // the 16 update warps
-      B2K_TACC(4, clock64() - t_w1);               // waiting for the slowest warp
-      if (warp == W_UPD0) B2K_TR(ti, 8);
       if (warp == W_UPD0 && lane == 0) {
         mbar_arrive(bar(G::B_LEMPTY + b));
         int s2 = xs;
@@ -846,11 +738,6 @@ k_fused_assign_update(const __grid_constant__ CUtensorMap mapX, const __grid_con
   }
 
   // ---- teardown ----
-  if (prof && lane == 0) {
-    long long* o = args.prof + ((size_t)blockIdx.x * NWARPS + warp) * 8;
-    o[0] = clock64() - t_role0;
-    for (int i = 0; i < 6; ++i) o[1 + i] = pw[i];
-  }
   tc_fence_before();
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -982,8 +869,7 @@ int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan
   plan->DP = in.DP;
   int64_t ntiles = (n + TM - 1) / TM;
   int grid = ctx->sm_count;
-  if (ctx->grid_limit > 0 && ctx->grid_limit < grid) grid = ctx->grid_limit;
-  plan->pair = (ctx->pair != 0 && in.KP == 64 && in.DP == 128) ? 1 : 0;
+  plan->pair = (in.KP == 64 && in.DP == 128) ? 1 : 0;   // the one CTA-pair (cta_group::2) instantiation
   if (plan->pair) {
     int64_t npairs = (ntiles + 1) / 2;
     grid &= ~1;
@@ -1050,24 +936,13 @@ int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int
   a.labels_out = labels_out;
   a.mind_out = mindist_out;
   a.do_update = do_update ? 1 : 0;
-  a.probe = ctx->probe;
   a.need_cost = (!do_update || mindist_out != nullptr) ? 1 : 0;
   a.st = st;
-  a.prof = nullptr;
-  if (ctx->profile_fused && !B2K_TRACE)
-    return b2k_fail(ctx, B2K_ERR_UNSUPPORTED, "profile_fused needs the diagnostic build (make trace; B2K_LIB=libb2kmeans_trace.so)");
-  if (ctx->profile_fused) {
-    if (!ctx->prof_dev) B2K_CUDA_OK(ctx, cudaMalloc(&ctx->prof_dev, (size_t)1024 * NWARPS * 8 * sizeof(long long)));
-    B2K_CUDA_OK(ctx, cudaMemsetAsync(ctx->prof_dev, 0, (size_t)(plan.grid + B2K_TRACE_CTAS) * NWARPS * 8 * sizeof(long long), s));
-    a.prof = ctx->prof_dev;
-    ctx->prof_grid = plan.grid + B2K_TRACE_CTAS;   // (+ trace area in diagnostic builds)
-  }
 
   int rc = B2K_ERR_UNSUPPORTED;
 #define B2K_DISPATCH(KP_, DP_) \
   if (!plan.pair && plan.KP == KP_ && plan.DP == DP_) rc = launch_inst<KP_, DP_, false>(ctx, plan.grid, mx, mh, ml, a, s);
   if (plan.pair && plan.KP == 64 && plan.DP == 128) rc = launch_inst<64, 128, true>(ctx, plan.grid, mx, mh, ml, a, s);
-  B2K_DISPATCH(64, 128)
   B2K_DISPATCH(64, 64)
   B2K_DISPATCH(64, 32)
   B2K_DISPATCH(32, 128)
@@ -1083,111 +958,5 @@ int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int
   B2K_TRY(rc);
   ctx->stats.kernel_launches++;
   ctx->stats.fused_tc_launches++;
-  return B2K_OK;
-}
-
-// diagnostics: per-role blocked-cycle counters of the last fused launch (option "profile_fused" = 1)
-extern "C" int b2k_get_fused_profile(b2k_ctx* ctx, long long* out, int64_t cap, int* grid_out, int* warps_out) {
-  if (!ctx || !out) return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_get_fused_profile: NULL argument");
-  if (!ctx->prof_dev || ctx->prof_grid == 0) return b2k_fail(ctx, B2K_ERR_STATE, "no fused profile recorded");
-  size_t cnt = (size_t)ctx->prof_grid * NWARPS * 8;
-  if ((int64_t)cnt > cap) return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_get_fused_profile: buffer too small");
-  B2K_CUDA_OK(ctx, cudaDeviceSynchronize());
-  B2K_CUDA_OK(ctx, cudaMemcpy(out, ctx->prof_dev, cnt * sizeof(long long), cudaMemcpyDeviceToHost));
-  if (grid_out) *grid_out = ctx->prof_grid;
-  if (warps_out) *warps_out = NWARPS;
-  return B2K_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// diagnostics: TMA streaming microbenchmark.  Persistent CTAs pull X through an nslot x 16 KB shared-memory
-// ring with the same 128B-swizzled [128 x 32 f32] boxes as the fused kernel; one consumer warp releases every
-// slot `hold` clock cycles after it lands.  Gives the bandwidth the ring can sustain as a function of its depth
-// and of how long the pipeline holds a slot (the fused kernel's ceiling; see DESIGN.md).
-// ------------------------------------------------------------------------------------------------
-namespace {
-__global__ void __launch_bounds__(1024, 1) k_tma_stream(const __grid_constant__ CUtensorMap mapX, int ntiles, int nch,
-                                                      int nslot, int hold, unsigned long long* sink, int box_rows) {
-  const int SLOT_BYTES = box_rows * CHUNK * 4;   // shadows the 16 KB constant: option "tma_box_rows" (diagnostic)
-  const int TM = box_rows;
-  extern __shared__ uint8_t smem_raw2[];
-  const uint32_t base = (smem_u32(smem_raw2) + 1023u) & ~1023u;
-  const uint32_t bars = base + (uint32_t)nslot * SLOT_BYTES;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < nslot; ++i) {
-      mbar_init(bars + 8u * i, 1);
-      mbar_init(bars + 8u * (nslot + i), 1);
-    }
-    mbar_init(bars + 8u * (2 * nslot), 1);        // "never" barrier: extra warps poll it (polling-load experiment)
-    *reinterpret_cast<volatile int*>(smem_raw2 + (base - smem_u32(smem_raw2)) + nslot * SLOT_BYTES + 8 * (2 * nslot + 2)) = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  volatile int* stop = reinterpret_cast<volatile int*>(smem_raw2 + (base - smem_u32(smem_raw2)) + nslot * SLOT_BYTES + 8 * (2 * nslot + 2));
-  int s = 0;
-  uint32_t ph = 0;
-  if (warp >= 2) {                                 // spinner warps
-    while (*stop == 0) { mbar_try_wait(bars + 8u * (2 * nslot), 0); }
-    return;
-  }
-  if (warp == 0) {
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x)
-      for (int c = 0; c < nch; ++c) {
-        mbar_wait(bars + 8u * (nslot + s), ph ^ 1u);
-        if (elect_one()) {
-          mbar_expect_tx(bars + 8u * s, SLOT_BYTES);
-          tma_load_2d(base + s * SLOT_BYTES, &mapX, bars + 8u * s, c * CHUNK, tile * TM);
-        }
-        __syncwarp();
-        if (++s == nslot) { s = 0; ph ^= 1u; }
-      }
-  } else {
-    unsigned long long acc = 0;
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x)
-      for (int c = 0; c < nch; ++c) {
-        mbar_wait(bars + 8u * s, ph);
-        if (hold > 0) {
-          const long long t0 = clock64();
-          while (clock64() - t0 < hold) {}
-        }
-        acc += lane;
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bars + 8u * (nslot + s));
-        if (++s == nslot) { s = 0; ph ^= 1u; }
-      }
-    if (acc == 0xdeadbeefULL) sink[0] = acc;
-    *stop = 1;
-  }
-}
-}  // namespace
-
-// out_ms receives the device time of one pass over X[n, d] (d multiple of 32) with the given ring depth / hold
-extern "C" int b2k_debug_tma_stream(b2k_ctx* ctx, const float* X, int64_t n, int d, int nslot, int hold_cycles,
-                                    float* out_ms) {
-  const int spinners = hold_cycles < 0 ? -hold_cycles : 0;   // hold < 0: |hold| extra warps polling an mbarrier
-  if (hold_cycles < 0) hold_cycles = 0;
-  const int box_rows = ctx->tma_box_rows > 0 ? ctx->tma_box_rows : TM;
-  if (!ctx || !X || !out_ms || d % CHUNK != 0 || nslot < 1 || nslot * box_rows > 13 * 128)
-    return b2k_fail(ctx, B2K_ERR_INVALID, "b2k_debug_tma_stream: bad argument");
-  CUtensorMap mx;
-  B2K_TRY(encode_2d(ctx, &mx, X, (uint64_t)d, (uint64_t)n, (uint64_t)d * 4, CHUNK, (uint32_t)box_rows, CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
-  const int smem = nslot * box_rows * CHUNK * 4 + 2 * nslot * 8 + 1024 + 128;
-  B2K_CUDA_OK(ctx, cudaFuncSetAttribute(k_tma_stream, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  B2K_TRY(b2k_scratch_reserve(ctx, 4096));
-  cudaEvent_t e0, e1;
-  B2K_CUDA_OK(ctx, cudaEventCreate(&e0));
-  B2K_CUDA_OK(ctx, cudaEventCreate(&e1));
-  const int ntiles = (int)((n + box_rows - 1) / box_rows);
-  for (int rep = 0; rep < 2; ++rep) {
-    if (rep == 1) B2K_CUDA_OK(ctx, cudaEventRecord(e0, 0));
-    k_tma_stream<<<ctx->sm_count, 64 + 32 * spinners, smem, 0>>>(mx, ntiles, d / CHUNK, nslot, hold_cycles,
-                                                 static_cast<unsigned long long*>(ctx->scratch), box_rows);
-  }
-  B2K_CUDA_OK(ctx, cudaEventRecord(e1, 0));
-  B2K_CUDA_OK(ctx, cudaEventSynchronize(e1));
-  B2K_CUDA_OK(ctx, cudaEventElapsedTime(out_ms, e0, e1));
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
   return B2K_OK;
 }

@@ -40,19 +40,12 @@ struct b2k_ctx {
   int kernel_path = B2K_PATH_AUTO;
   int time_kernels = 0;
   int check_every = 4;
-  int grid_limit = 0;
-  int probe = 0;                 // debug/experiment switch for the fused kernel (0 = normal)
-  int pair = 1;                  // option "pair": use the cta_group::2 instantiation where available (default on)
   int adaptive_path = 1;         // option "adaptive_path": a Lloyd loop on the large-shape kernel falls back to the generic
                                  // kernels for its remaining iterations when most rows need the exact fix-up
   int force_variant_t = 0;       // option "variant_t": route every supported shape through b2k_fused_t.cu (tests)
-  int tma_box_rows = 0;          // option "tma_box_rows": rows per TMA box of b2k_debug_tma_stream (diagnostic; 0 = 128)
   int collect_recheck = 0;       // option "collect_recheck": fill stats.recheck_* (costs a stream sync per call)
-  int profile_fused = 0;         // record per-role blocked-cycle counters of the fused kernel
   void* xnorm_cache = nullptr;   // float2 [xnorm_cache_rows]: row norms shared by the passes of one fit (B2kNormScope)
   int64_t xnorm_cache_rows = 0;
-  long long* prof_dev = nullptr;  // [grid][18 warps][8]
-  int prof_grid = 0;
   // comm
   B2kNccl* nccl = nullptr;
   int nranks = 1;

@@ -44,14 +44,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   }
 }
 
-// optional stage profiling (FusedArgs::prof != NULL): cycles spent blocked on a barrier are added to `acc`
-__device__ __forceinline__ void mbar_wait_p(uint32_t bar, uint32_t parity, bool prof, long long& acc) {
-  if (!prof) { mbar_wait(bar, parity); return; }
-  long long t0 = clock64();
-  mbar_wait(bar, parity);
-  acc += clock64() - t0;
-}
-
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int x, int y) {
   asm volatile(
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
@@ -184,41 +176,6 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t rank)
   // this side, tcgen05.fence::after_thread_sync on the consumer side), not generic-proxy memory — a cluster-scope
   // release here costs several hundred cycles per hand-off (measured).
   asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity), "r"(200000u)
-      : "memory");
-  return ok;
-}
-// Dedicated single-warp poller (the MMA issuer): non-blocking test in a tight loop, CTA-scope acquire.  What these
-// waits order is TMEM traffic (tcgen05 fences on both sides), and the phase flips in this CTA's own shared memory
-// whoever arrives.  Kept as an alternative to mbar_wait_cluster (B2K_MMA_WAIT): same step time, measured.
-__device__ __forceinline__ void mbar_spin(uint32_t bar, uint32_t parity) {
-  uint32_t spins = 0;
-  for (;;) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (ok) return;
-    if (++spins == (1u << 24)) mbar_timeout(bar, parity);
-  }
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
-    if (++spins == (1u << 22)) mbar_timeout(bar, parity);
-  }
 }
 __device__ __forceinline__ void tc_commit_pair(uint32_t bar) {   // signals the barrier at this offset in BOTH CTAs
   asm volatile(
