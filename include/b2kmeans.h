@@ -116,8 +116,7 @@ int b2k_ctx_create(int device, b2k_ctx** out);
 int b2k_ctx_destroy(b2k_ctx* ctx);
 /* Options: "kernel_path" (b2k_kernel_path), "time_kernels" (0/1/2: CUDA events around every fused launch; 2 = also
  * around the partial fold, the allreduce and finalize), "check_every" (iterations between host
- * convergence polls, default 4), "variant_t" (1 = route every shape with k, d <= 256 through the
- * large-shape kernel b2k_fused_t.cu; default 0 = only shapes the 3xTF32 kernel does not cover), "collect_recheck"
+ * convergence polls, default 4), "collect_recheck"
  * (1 = lloyd/assign synchronise and fill b2k_stats.recheck_*), "adaptive_path" (see b2k_stats.path_switch_iter), "ingest_threads" (host threads of the pageable -> pinned
  * staging copy of b2k_ingest_append; 0 = default: 4, capped by half of the CPUs the process may use).  Any other key
  * fails with B2K_ERR_INVALID. */

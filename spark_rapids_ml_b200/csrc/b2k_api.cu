@@ -95,8 +95,6 @@ extern "C" int b2k_ctx_set_option(b2k_ctx* ctx, const char* key, int64_t value) 
     ctx->check_every = (int)value;
   } else if (k == "adaptive_path") {
     ctx->adaptive_path = value ? 1 : 0;
-  } else if (k == "variant_t") {
-    ctx->force_variant_t = value ? 1 : 0;
   } else if (k == "ingest_threads") {
     if (value < 0 || value > 64) return b2k_fail(ctx, B2K_ERR_INVALID, "ingest_threads must be in [0, 64]");
     b2k_copy_pool_destroy(ctx);
@@ -161,21 +159,6 @@ int check_shape(b2k_ctx* ctx, const char* who, const void* X, int64_t n, int d, 
   return B2K_OK;
 }
 
-// `path`: the kernel path the pass honours (B2K_PATH_*)
-bool want_fused(b2k_ctx* ctx, int path, int64_t n, int d, int k, const float* X, int* status) {
-  *status = B2K_OK;
-  bool ok = b2k_fused_supported(ctx, n, d, k, X);
-  if (path == B2K_PATH_GENERIC) return false;
-  if (path == B2K_PATH_TCGEN05 && !ok) {
-    *status = b2k_fail(ctx, B2K_ERR_UNSUPPORTED,
-                       "kernel_path=tcgen05 requested but shape (n=" + std::to_string(n) + ", d=" +
-                           std::to_string(d) + ", k=" + std::to_string(k) +
-                           ") is outside the fused kernel's instantiations");
-    return false;
-  }
-  return ok;
-}
-
 // Scratch of one Lloyd loop.
 struct LoopBuffers {
   B2kLoopState* st;
@@ -194,51 +177,85 @@ struct LoopBuffers {
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
-// Chunked assignment for cluster counts beyond one fused pass: the centres are cut into chunks of exactly CH (the last
-// chunk is [k - CH, k): the overlap is harmless for a min), each chunk runs one fused assign pass that yields the min
-// distance and label of every row within the chunk, and k_merge_chunk keeps the smaller distance (strict '<': lowest
-// cluster index on ties).  d <= 128: CH = 128 through the 3xTF32 kernel (exact, no fix-up); 128 < d <= 256: CH = 256
-// through the large-shape kernel (1xTF32 screening + exact fix-up).  Used for k > 256 (assign passes, and Lloyd with the
-// generic label-driven update) and — d <= 128 only — for k > 128 when the caller expects near-ties (the k-means||
-// candidate passes: candidates drawn from one blob are almost equidistant from its rows, which is the worst case of
-// the screening kernel and free for the 3xTF32 one).  Replaces the SIMT assign of the generic path for d % 4 == 0.
+// Which kernels a pass over X[n, d] against k centres runs.  TMA-ok: d % 4 == 0, X 16-byte aligned and
+// 1 <= n <= 0x7fffff00.  tc(d, k): a 3xTF32 instantiation with DP = d rounded up to a multiple of 32 (96 -> 128) and
+// KP >= k exists (b2k_fused_tc_inst: DP 32 with KP 16/32/64, DP 64 and 128 with KP 16/32/64/128).
+//
+//   kernel_path      condition (first match wins)                              pass runs on
+//   generic          any                                                       generic
+//   auto / tcgen05   TMA-ok, d <= 256, and either k > 256, or (near_tie,       chunks of ch = 128 (d <= 128) or 256
+//                    d <= 128, k > 128)                                        centres: each chunk on variant 0 if
+//                                                                              tc(d, ch), otherwise variant 1
+//   auto / tcgen05   TMA-ok and tc(d, k)                                       variant 0; CTA pairs iff KP = 64, DP = 128
+//   auto / tcgen05   TMA-ok, d <= 256, k <= 256                                variant 1, DP = 128 (d <= 128) or 256
+//   auto             otherwise (this includes n = 0 in a Lloyd loop)           generic
+//   tcgen05          otherwise                                                 B2K_ERR_UNSUPPORTED
+//
+// Variant 0 is the 3xTF32 kernel (b2k_fused_tc.cu), variant 1 the 1xTF32 screening kernel with its exact fix-up
+// (b2k_fused_t.cu).  So d <= 32 with 64 < k <= 128, and 128-centre chunks at d <= 32, run on the screening kernel.
+//
+// Chunks: the centres are cut into chunks of exactly ch (the last chunk is [k - ch, k): the overlap is harmless for a
+// min), each chunk runs one fused assign pass that yields the min distance and label of every row within the chunk, and
+// k_merge_chunk keeps the smaller distance (strict '<': lowest cluster index on ties).  A chunked Lloyd loop keeps the
+// generic label-driven update.  near_tie is set by the k-means|| candidate passes: candidates drawn from one blob are
+// almost equidistant from its rows, which is the worst case of the screening kernel, so they prefer 128-centre chunks.
 // ------------------------------------------------------------------------------------------------
+int b2k_choose_kernel(b2k_ctx* ctx, int path, bool near_tie, int64_t n, int d, int k, const float* X, B2kChoice* out) {
+  B2kChoice c;
+  const bool tma_ok = d % 4 == 0 && (reinterpret_cast<uintptr_t>(X) & 15u) == 0 && n >= 1 && n <= (int64_t)0x7fffff00;
+  if (path != B2K_PATH_GENERIC && tma_ok && d <= kFusedTMaxD) {
+    if (k > kFusedTMaxK || (near_tie && d <= 128 && k > 128)) {
+      c.kind = B2kChoice::CHUNKED;
+      c.ch = d <= 128 ? 128 : 256;
+    } else if (k <= kFusedTMaxK) {
+      c.kind = B2kChoice::FUSED;
+    }
+  }
+  if (c.kind != B2kChoice::GENERIC) {
+    const int kk = c.kind == B2kChoice::CHUNKED ? c.ch : k;
+    if (b2k_fused_tc_inst(d, kk, &c.KP, &c.DP)) {
+      c.pair = b2k_tc_pair(c.KP, c.DP) ? 1 : 0;
+    } else {
+      c.variant = 1;
+      c.KP = kFusedTMaxK;
+      c.DP = d <= 128 ? 128 : 256;
+      c.pair = 1;
+    }
+  } else if (path == B2K_PATH_TCGEN05) {
+    return b2k_fail(ctx, B2K_ERR_UNSUPPORTED,
+                    "kernel_path=tcgen05 requested but shape (n=" + std::to_string(n) + ", d=" + std::to_string(d) +
+                        ", k=" + std::to_string(k) + ") is outside the fused kernel's instantiations");
+  }
+  *out = c;
+  return B2K_OK;
+}
+
 namespace {
 struct ChunkedAssign {
-  B2kFusedPlan plan;
-  int ch = 0;                // chunk size
+  B2kFusedPlan plan;         // the kernel of one chunk (plan.choice.ch centres)
   int32_t* tmp_lab = nullptr;
   float* tmp_md = nullptr;
   int32_t* lab_acc = nullptr;   // used when the caller passes no labels / mindist buffer
   float* md_acc = nullptr;
 };
-// chunk size, 0 = this (d, k) is not chunked.  `path`: the kernel path the pass honours; `near_tie`: the caller expects
-// near-ties (prefer exact 128-centre chunks, d <= 128).
-int chunked_assign_ch(const b2k_ctx* ctx, int path, bool near_tie, int64_t n, int d, int k, const float* X) {
-  if (path == B2K_PATH_GENERIC || n <= 0 || d > 256) return 0;
-  const int ch = (d <= 128 && !ctx->force_variant_t) ? 128 : 256;
-  const bool want = k > 256 || (ch == 128 && k > 128 && near_tie);
-  if (!want || !b2k_fused_supported(ctx, n, d, ch, X)) return 0;
-  return ch;
-}
 // the caller runs b2k_fused_prepare(ca.plan, ...) before chunked_assign_run
-int chunked_assign_layout(b2k_ctx* ctx, int64_t n, int d, int ch, Arena& A, ChunkedAssign* ca) {
-  ca->ch = ch;
+int chunked_assign_layout(b2k_ctx* ctx, const B2kChoice& c, int64_t n, int d, Arena& A, ChunkedAssign* ca) {
   ca->tmp_lab = A.take<int32_t>(n);
   ca->tmp_md = A.take<float>(n);
   ca->lab_acc = A.take<int32_t>(n);
   ca->md_acc = A.take<float>(n);
-  return b2k_fused_plan(ctx, n, d, ch, A, &ca->plan);
+  return b2k_fused_plan(ctx, c, n, d, c.ch, A, &ca->plan);
 }
 int chunked_assign_run(b2k_ctx* ctx, const ChunkedAssign& ca, const float* X, int64_t n, int d, const float* C, int k,
                        int32_t* labels, float* mindist, const B2kLoopState* st, cudaStream_t s) {
   int32_t* lab = labels ? labels : ca.lab_acc;
   float* md = mindist ? mindist : ca.md_acc;
-  for (int c0 = 0; c0 < k; c0 += ca.ch) {
-    const int base = std::min(c0, k - ca.ch);
+  const int ch = ca.plan.choice.ch;
+  for (int c0 = 0; c0 < k; c0 += ch) {
+    const int base = std::min(c0, k - ch);
     const bool first = c0 == 0;
     // every chunk writes mindist, which makes both variants compute the cost: the merge needs no cost partials
-    B2K_TRY(b2k_launch_fused(ctx, ca.plan, X, n, d, C + (size_t)base * d, ca.ch, first ? lab : ca.tmp_lab,
+    B2K_TRY(b2k_launch_fused(ctx, ca.plan, X, n, d, C + (size_t)base * d, ch, first ? lab : ca.tmp_lab,
                              first ? md : ca.tmp_md, false, false, st, s));
     if (!first) B2K_TRY(b2k_launch_merge_chunk(ctx, md, lab, ca.tmp_md, ca.tmp_lab, base, n, st, s));
   }
@@ -253,36 +270,31 @@ int chunked_assign_run(b2k_ctx* ctx, const ChunkedAssign& ca, const float* X, in
 static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, float* C, int max_iter, double tol,
                       B2kNormScope* norms, int* n_iter_out, double* shift_out, int* path_out, cudaStream_t s) {
   if (max_iter < 0) return b2k_fail(ctx, B2K_ERR_INVALID, "lloyd: max_iter < 0");
-  const int path = ctx->kernel_path;
-  // k > 256 (d <= 256): the assignment runs in 256-centre chunks on the large-shape kernel, the update stays generic
-  const int chunk_ch = k > 256 ? chunked_assign_ch(ctx, path, false, n, d, k, X) : 0;
-  const bool chunked = chunk_ch != 0;
-  int st_rc = B2K_OK;
-  const bool fused = chunked ? false : want_fused(ctx, path, n, d, k, X, &st_rc);
-  B2K_TRY(st_rc);
-  ctx->stats.last_path = (fused || chunked) ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
+  B2kChoice c;
+  B2K_TRY(b2k_choose_kernel(ctx, ctx->kernel_path, false, n, d, k, X, &c));
+  const bool fused = c.kind == B2kChoice::FUSED;
+  const bool chunked = c.kind == B2kChoice::CHUNKED;
+  // The large-shape kernel (1xTF32 screening) hands near-tie rows to an exact fix-up; on data where most rows are
+  // near-ties (e.g. uniform noise in 256 dimensions) the generic kernels are several times faster, so the loop may
+  // switch to them between bursts.  The choice is local to the rank: both paths fill the same R buffer.
+  const bool can_switch = fused && c.variant == 1 && ctx->adaptive_path && ctx->kernel_path == B2K_PATH_AUTO;
 
   LoopBuffers B{};
   ChunkedAssign ca;
-  bool can_switch = false;
   const size_t rlen = b2k_reduced_len(k, d);
   B2K_TRY(carve_scratch(ctx, [&](Arena& A) -> int {
     B.st = A.take<B2kLoopState>(1);
     B.R = A.take<double>(rlen);
     B.shift_scratch = A.take<double>(k);
     B.cnorm = A.take<float>(k);
-    if (fused) B2K_TRY(b2k_fused_plan(ctx, n, d, k, A, &B.plan));
-    // The large-shape kernel (1xTF32 screening) hands near-tie rows to an exact fix-up; on data where most rows are
-    // near-ties (e.g. uniform noise in 256 dimensions) the generic kernels are several times faster, so the loop may
-    // switch to them between bursts.  The choice is local to the rank: both paths fill the same R buffer.
-    can_switch = fused && B.plan.variant == 1 && ctx->adaptive_path && path == B2K_PATH_AUTO;
+    if (fused) B2K_TRY(b2k_fused_plan(ctx, c, n, d, k, A, &B.plan));
     if (!fused || can_switch) {
-      b2k_update_generic_scratch(ctx, n, d, k, &B.P);
+      B.P = b2k_update_generic_slots(ctx, n, d, k);
       B.labels = A.take<int32_t>(n > 0 ? n : 1);
       B.partials = A.take<float>((size_t)B.P * k * d);
       B.counts = A.take<int32_t>((size_t)B.P * k);
     }
-    if (chunked) B2K_TRY(chunked_assign_layout(ctx, n, d, chunk_ch, A, &ca));
+    if (chunked) B2K_TRY(chunked_assign_layout(ctx, c, n, d, A, &ca));
     return B2K_OK;
   }));
 
@@ -419,7 +431,7 @@ static int lloyd_impl(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, flo
     cudaEventDestroy(loop1);
   }
   ctx->stats.last_n_iter = ctx->h_state->iter;
-  ctx->stats.last_path = (fused_now || chunked) ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
+  ctx->stats.last_path = ctx->stats.path_switch_iter >= 0 ? B2K_PATH_GENERIC : c.path();
   if (path_out) *path_out = ctx->stats.last_path;
   if (fused && ctx->collect_recheck && max_iter > 0) {
     unsigned long long rs[2];
@@ -448,16 +460,15 @@ namespace {
 // per-call choices of an assign pass
 struct PassOpts {
   int path;                        // kernel path to honour (B2K_PATH_*): the option, or the path a fit's Lloyd loop ended on
-  bool near_tie = false;           // the caller expects near-ties (chunked_assign_ch)
+  bool near_tie = false;           // the caller expects near-ties (b2k_choose_kernel)
   B2kNormScope* norms = nullptr;   // the fit's row-norm scope, for passes over the fit's X
 };
 
 constexpr int kCostBlocks = 1024;   // block sums of a cost formed from mindist
 
-// One assign pass: chunked (ch > 0), one fused pass, or the generic kernels, and the scratch that route takes.
+// One assign pass: chunked, one fused pass, or the generic kernels, and the scratch that route takes.
 struct AssignPass {
-  int ch = 0;
-  bool fused = false;
+  B2kChoice c;
   ChunkedAssign ca;
   B2kFusedPlan plan;
   float* cnorm = nullptr;    // generic
@@ -467,15 +478,13 @@ struct AssignPass {
 
 int assign_layout(b2k_ctx* ctx, const PassOpts& o, const float* X, int64_t n, int d, int k, bool own_md, Arena& A,
                   AssignPass* p) {
-  if ((p->ch = chunked_assign_ch(ctx, o.path, o.near_tie, n, d, k, X))) {
-    B2K_TRY(chunked_assign_layout(ctx, n, d, p->ch, A, &p->ca));
+  B2K_TRY(b2k_choose_kernel(ctx, o.path, o.near_tie, n, d, k, X, &p->c));
+  if (p->c.kind == B2kChoice::CHUNKED) {
+    B2K_TRY(chunked_assign_layout(ctx, p->c, n, d, A, &p->ca));
     p->blocks = A.take<double>(kCostBlocks);
     return B2K_OK;
   }
-  int rc;
-  p->fused = want_fused(ctx, o.path, n, d, k, X, &rc);
-  B2K_TRY(rc);
-  if (p->fused) return b2k_fused_plan(ctx, n, d, k, A, &p->plan);
+  if (p->c.kind == B2kChoice::FUSED) return b2k_fused_plan(ctx, p->c, n, d, k, A, &p->plan);
   p->cnorm = A.take<float>(k);
   if (own_md) p->md = A.take<float>(n > 0 ? n : 1);
   p->blocks = A.take<double>(kCostBlocks);
@@ -505,13 +514,13 @@ static int assign_impl(b2k_ctx* ctx, Arena A, const PassOpts& o, const float* X,
   AssignPass p;
   B2K_TRY(assign_layout(ctx, o, X, n, d, k, cost_dev && !mindist, A, &p));
   if (A.overflow) return b2k_fail(ctx, B2K_ERR_STATE, "assign_impl: the pass outgrows the scratch reserved for it");
-  ctx->stats.last_path = (p.ch || p.fused) ? B2K_PATH_TCGEN05 : B2K_PATH_GENERIC;
-  if (p.ch) {   // chunks of ch centres through a fused assign pass each
+  ctx->stats.last_path = p.c.path();
+  if (p.c.kind == B2kChoice::CHUNKED) {   // chunks of ch centres through a fused assign pass each
     B2K_TRY(b2k_fused_prepare(ctx, p.ca.plan, X, n, d, o.norms, s));
     B2K_TRY(chunked_assign_run(ctx, p.ca, X, n, d, C, k, labels, mindist, nullptr, s));
     if (cost_dev)
       B2K_TRY(b2k_launch_sum_f32_to_f64(ctx, mindist ? mindist : p.ca.md_acc, n, cost_dev, p.blocks, kCostBlocks, s));
-  } else if (p.fused) {
+  } else if (p.c.kind == B2kChoice::FUSED) {
     B2K_TRY(b2k_fused_prepare(ctx, p.plan, X, n, d, o.norms, s));
     B2K_TRY(b2k_launch_fused(ctx, p.plan, X, n, d, C, k, labels, mindist, false, cost_dev != nullptr, nullptr, s));
     // fold the per-CTA cost partials in index order
@@ -522,9 +531,9 @@ static int assign_impl(b2k_ctx* ctx, Arena A, const PassOpts& o, const float* X,
     B2K_TRY(b2k_launch_assign_generic(ctx, X, n, d, C, p.cnorm, k, labels, md, nullptr, s));
     if (cost_dev) B2K_TRY(b2k_launch_sum_f32_to_f64(ctx, md, n, cost_dev, p.blocks, kCostBlocks, s));
   }
-  if (ctx->collect_recheck && (p.ch || p.fused)) {
+  if (ctx->collect_recheck && p.c.kind != B2kChoice::GENERIC) {
     unsigned long long rs[2];
-    B2K_TRY(b2k_fused_recheck_stats(ctx, p.ch ? p.ca.plan : p.plan, rs, s));
+    B2K_TRY(b2k_fused_recheck_stats(ctx, p.c.kind == B2kChoice::CHUNKED ? p.ca.plan : p.plan, rs, s));
     ctx->stats.recheck_rows = (int64_t)rs[0];
     ctx->stats.recheck_candidates = (int64_t)rs[1];
   }
@@ -693,7 +702,7 @@ static int init_random(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, ui
 // (clustering.py:134-136).  Distributional parity only (the reference's own seeded test is xfail).
 static int init_kmeans_parallel(b2k_ctx* ctx, const float* X, int64_t n, int d, int k, uint64_t seed,
                                 double oversampling, B2kNormScope* norms, float* C, cudaStream_t s) {
-  // the candidate passes are near-tie heavy (see chunked_assign_ch); only those over X share the fit's row norms
+  // the candidate passes are near-tie heavy (see b2k_choose_kernel); only those over X share the fit's row norms
   const PassOpts ox{ctx->kernel_path, true, norms};
   const PassOpts ocand{ctx->kernel_path, true, nullptr};
   const int rounds = 5;

@@ -16,13 +16,13 @@
 //     DEFERRED: the epilogue appends it (row id + the bit mask of every cluster within thr of the best = its
 //     candidates) to the CTA pair's segment of a fix-up list and publishes no label for it, so the pass never
 //     waits for an exact evaluation.  k_fix_labels_t then decides those rows exactly (fp32 dot products against the
-//     fp32 centres, ascending cluster order, strict '<' = lowest index on ties) and k_fix_accum_t adds them to one
-//     extra partial-sum slot (fixed list order: deterministic).  Rows outside the bound provably have the same
-//     argmin in exact arithmetic, so labels match the 3xTF32 / fp32 path.
+//     fp32 centres, ascending cluster order, strict '<' = lowest index on ties) and k_fix_accum_t adds them to
+//     FIX_SLOTS = 4 extra partial-sum slots (slot q: the segments q mod 4, fixed list order: deterministic).  Rows
+//     outside the bound provably have the same argmin in exact arithmetic, so labels match the 3xTF32 / fp32 path.
 //   * update: per-cluster sums live in REGISTERS, one [256, 256] accumulator set per CTA PAIR (each CTA: 128
-//     clusters x 256 columns = 64 registers per update thread).  Rows are counting-sorted by (owner warp, cluster,
-//     row) as in b2k_fused_tc.cu; a warp reads its rows from the local ring or, for the peer's rows, through
-//     DSMEM (ld.shared::cluster).  No atomics; static schedule; deterministic.
+//     clusters x 256 columns = 64 registers per update thread).  Each update warp finds its rows itself from the
+//     labels the epilogue publishes (through the cluster -> warp table of k_tables_t) and reads them from the local
+//     ring or, for the peer's rows, through DSMEM (ld.shared::cluster).  No atomics; static schedule; deterministic.
 //   * assign / inertia passes (UPD = false): the same screening + recheck for the labels; the "update" warps
 //     compute the exact min distance sum (x - c)^2 of every row from the tile in shared memory.
 //
@@ -1000,7 +1000,7 @@ __global__ void __launch_bounds__(256) k_fix_accum_t(const FixArgs f) {
 // host side
 // ------------------------------------------------------------------------------------------------
 void t_layout(B2kFusedPlan* p, int64_t n, int k, int d, Arena& A) {
-  p->ct = A.take<float>((size_t)256 * p->DP, 1024);
+  p->ct = A.take<float>((size_t)256 * p->choice.DP, 1024);
   p->cnorm = A.take<float>(512);
   p->thr = A.take<float>(4);
   p->keytab = A.take<uint8_t>(512);
@@ -1031,19 +1031,7 @@ int launch_t(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const TArgs& a, cuda
 }
 }  // namespace
 
-bool b2k_fused_t_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X) {
-  (void)ctx;
-  if (n < 1 || n > (int64_t)0x7fffff00 * 1LL) return false;
-  if (d % 4 != 0 || d > 256 || k > 256) return false;
-  if ((reinterpret_cast<uintptr_t>(X) & 15u) != 0) return false;
-  return true;
-}
-
 int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan) {
-  plan->variant = 1;
-  plan->KP = 256;
-  plan->DP = d <= 128 ? 128 : 256;
-  plan->pair = 1;
   const int64_t nsteps = (n + TN - 1) / TN;
   int grid = ctx->sm_count & ~1;
   if (nsteps * 2 < grid) grid = (int)nsteps * 2;
@@ -1088,13 +1076,14 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, i
   uint8_t* keytab = plan.keytab;
   const int npairs = plan.grid / 2;
 
-  k_prep_centers_t<<<32, 256, 0, s>>>(C, k, d, plan.DP, plan.ct, cnorm, st);
+  k_prep_centers_t<<<32, 256, 0, s>>>(C, k, d, plan.choice.DP, plan.ct, cnorm, st);
   k_tables_t<<<1, 256, 0, s>>>(do_update ? prev_counts : nullptr, k, cnorm, keytab, keytab + 256, plan.thr, st);
   ctx->stats.kernel_launches += 2;
   B2K_CUDA_OK(ctx, cudaGetLastError());
 
   CUtensorMap mx;
-  B2K_TRY(b2k_fused_encode_2d(ctx, &mx, X, (uint64_t)d, (uint64_t)n, (uint64_t)d * 4, CHUNK, TNH, 1));
+  B2K_TRY(b2k_encode_2d(ctx, &mx, X, (uint64_t)d, (uint64_t)n, (uint64_t)d * 4, CHUNK, TNH,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
 
   TArgs a{};
   a.n = n;
@@ -1124,7 +1113,7 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, i
   if (npairs > FIX_MAXP) return b2k_fail(ctx, B2K_ERR_STATE, "fused_t: more CTA pairs than the fix-up kernels index");
 
   int rc;
-  if (plan.DP == 128) rc = do_update ? launch_t<4, true>(ctx, plan.grid, mx, a, s) : launch_t<4, false>(ctx, plan.grid, mx, a, s);
+  if (plan.choice.DP == 128) rc = do_update ? launch_t<4, true>(ctx, plan.grid, mx, a, s) : launch_t<4, false>(ctx, plan.grid, mx, a, s);
   else rc = do_update ? launch_t<8, true>(ctx, plan.grid, mx, a, s) : launch_t<8, false>(ctx, plan.grid, mx, a, s);
   B2K_TRY(rc);
   ctx->stats.kernel_launches++;

@@ -776,8 +776,10 @@ int get_encoder(b2k_ctx* ctx, EncodeTiledFn* fn) {
   return B2K_OK;
 }
 
-int encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,
-              uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer, CUtensorMapL2promotion l2) {
+}  // namespace
+
+int b2k_encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,
+                  uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer, CUtensorMapL2promotion l2) {
   EncodeTiledFn fn;
   B2K_TRY(get_encoder(ctx, &fn));
   cuuint64_t dims[2] = {inner, outer};
@@ -791,36 +793,31 @@ int encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, 
   return B2K_OK;
 }
 
-}  // namespace
-int b2k_fused_encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,
-                        uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer, int l2_256) {
-  return encode_2d(ctx, map, base, inner, outer, row_stride_bytes, box_inner, box_outer,
-                   l2_256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
-}
 namespace {
+// The 3xTF32 instantiations compiled into the library, as <KP, DP>.  b2k_fused_tc_inst searches this list and
+// b2k_launch_fused dispatches over it; b2k_tc_pair picks the one that runs on CTA pairs.  There is no <128, 32>:
+// d <= 32 with k > 64 runs on the screening kernel (DESIGN.md 4.1).
+template <int KP_, int DP_>
 struct Inst {
-  int KP, DP;
+  static constexpr int KP = KP_, DP = DP_;
 };
-// instantiations compiled into the library
-constexpr Inst kInst[] = {{64, 128}, {64, 64}, {64, 32}, {32, 128}, {128, 128}, {128, 64}, {16, 32}, {16, 64}, {32, 64}, {32, 32}, {16, 128}};
+template <typename... I>
+struct InstList {};
+using Insts = InstList<Inst<16, 32>, Inst<32, 32>, Inst<64, 32>,
+                       Inst<16, 64>, Inst<32, 64>, Inst<64, 64>, Inst<128, 64>,
+                       Inst<16, 128>, Inst<32, 128>, Inst<64, 128>, Inst<128, 128>>;
 
-bool pick_inst(int d, int k, Inst* out) {
-  int DP = (d + CHUNK - 1) / CHUNK * CHUNK;
-  if (DP == 96) DP = 128;
-  int best = -1;
-  for (size_t i = 0; i < sizeof(kInst) / sizeof(kInst[0]); ++i) {
-    if (kInst[i].DP == DP && kInst[i].KP >= k) {
-      if (best < 0 || kInst[i].KP < kInst[best].KP) best = (int)i;
-    }
-  }
-  if (best < 0) return false;
-  *out = kInst[best];
-  return true;
+template <typename... I>
+int smallest_kp(InstList<I...>, int DP, int k) {
+  int kp = 0;
+  ((I::DP == DP && I::KP >= k && (kp == 0 || I::KP < kp) ? (void)(kp = I::KP) : (void)0), ...);
+  return kp;
 }
 
-template <int KP, int DP, bool PAIR, bool NC>
+template <int KP, int DP, bool NC>
 int launch_inst_nc(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const CUtensorMap& mh, const CUtensorMap& ml,
                 const FusedArgs& a, cudaStream_t s) {
+  constexpr bool PAIR = b2k_tc_pair(KP, DP);
   using G = Cfg<KP, DP, PAIR>;
   auto kern = k_fused_assign_update<KP, DP, PAIR, NC>;
   B2K_CUDA_OK(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM_BYTES));
@@ -830,17 +827,27 @@ int launch_inst_nc(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const CUtensor
   return B2K_OK;
 }
 
-template <int KP, int DP, bool PAIR>
+template <int KP, int DP>
 int launch_inst(b2k_ctx* ctx, int grid, const CUtensorMap& mx, const CUtensorMap& mh, const CUtensorMap& ml,
                 const FusedArgs& a, cudaStream_t s) {
-  return a.need_cost ? launch_inst_nc<KP, DP, PAIR, true>(ctx, grid, mx, mh, ml, a, s)
-                     : launch_inst_nc<KP, DP, PAIR, false>(ctx, grid, mx, mh, ml, a, s);
+  return a.need_cost ? launch_inst_nc<KP, DP, true>(ctx, grid, mx, mh, ml, a, s)
+                     : launch_inst_nc<KP, DP, false>(ctx, grid, mx, mh, ml, a, s);
+}
+
+// launches the listed instantiation <KP, DP>; B2K_ERR_UNSUPPORTED when it is not listed
+template <typename... I>
+int launch_listed(InstList<I...>, int KP, int DP, b2k_ctx* ctx, int grid, const CUtensorMap& mx,
+                  const CUtensorMap& mh, const CUtensorMap& ml, const FusedArgs& a, cudaStream_t s) {
+  int rc = B2K_ERR_UNSUPPORTED;
+  (void)(((I::KP == KP && I::DP == DP) && (rc = launch_inst<I::KP, I::DP>(ctx, grid, mx, mh, ml, a, s), true)) || ...);
+  return rc;
 }
 
 void plan_layout(B2kFusedPlan* p, int k, int d, Arena& A) {
-  p->c_hi = A.take<float>((size_t)p->KP * p->DP, 1024);
-  p->c_lo = A.take<float>((size_t)p->KP * p->DP);
-  p->cnorm = A.take<float>(p->KP);
+  const int KP = p->choice.KP, DP = p->choice.DP;
+  p->c_hi = A.take<float>((size_t)KP * DP, 1024);
+  p->c_lo = A.take<float>((size_t)KP * DP);
+  p->cnorm = A.take<float>(KP);
   p->keytab = A.take<uint8_t>(512);
   p->partials = A.take<float>((size_t)p->grid * k * d);
   p->counts = A.take<int32_t>((size_t)p->grid * k);
@@ -848,29 +855,22 @@ void plan_layout(B2kFusedPlan* p, int k, int d, Arena& A) {
 }
 }  // namespace
 
-bool b2k_fused_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X) {
-  (void)ctx;
-  if (n < 1 || n > (int64_t)0x7fffff00 * 1LL) return false;
-  if (d % 4 != 0) return false;                                   // TMA: row pitch must be a multiple of 16 B
-  if ((reinterpret_cast<uintptr_t>(X) & 15u) != 0) return false;  // TMA: 16 B aligned base
-  Inst in;
-  if (pick_inst(d, k, &in)) return true;
-  return b2k_fused_t_supported(ctx, n, d, k, X);   // large shapes: b2k_fused_t.cu (k <= 256, d <= 256)
+bool b2k_fused_tc_inst(int d, int k, int* KP, int* DP) {
+  int dp = (d + CHUNK - 1) / CHUNK * CHUNK;
+  if (dp == 96) dp = 128;
+  const int kp = smallest_kp(Insts{}, dp, k);
+  if (kp == 0) return false;
+  *KP = kp;
+  *DP = dp;
+  return true;
 }
 
-int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan) {
-  Inst in;
-  if (!pick_inst(d, k, &in) || ctx->force_variant_t) {
-    if (d % 4 == 0 && d <= 256 && k <= 256) return b2k_fused_t_plan(ctx, n, d, k, A, plan);
-    return b2k_fail(ctx, B2K_ERR_UNSUPPORTED, "fused kernel: no instantiation for this (k, d)");
-  }
-  plan->variant = 0;
-  plan->KP = in.KP;
-  plan->DP = in.DP;
+int b2k_fused_plan(b2k_ctx* ctx, const B2kChoice& c, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan) {
+  plan->choice = c;
+  if (c.variant == 1) return b2k_fused_t_plan(ctx, n, d, k, A, plan);
   int64_t ntiles = (n + TM - 1) / TM;
   int grid = ctx->sm_count;
-  plan->pair = (in.KP == 64 && in.DP == 128) ? 1 : 0;   // the one CTA-pair (cta_group::2) instantiation
-  if (plan->pair) {
+  if (c.pair) {
     int64_t npairs = (ntiles + 1) / 2;
     grid &= ~1;
     if (npairs * 2 < grid) grid = (int)npairs * 2;
@@ -888,13 +888,13 @@ int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan
 
 int b2k_fused_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
                       cudaStream_t s) {
-  if (plan.variant == 1) return b2k_fused_t_prepare(ctx, plan, X, n, d, norms, s);
+  if (plan.choice.variant == 1) return b2k_fused_t_prepare(ctx, plan, X, n, d, norms, s);
   return B2K_OK;
 }
 
 int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, unsigned long long out[2], cudaStream_t s) {
   out[0] = out[1] = 0ull;
-  if (plan.variant != 1) return B2K_OK;
+  if (plan.choice.variant != 1) return B2K_OK;
   B2K_CUDA_OK(ctx, cudaMemcpyAsync(out, plan.rstat, 16, cudaMemcpyDeviceToHost, s));
   B2K_CUDA_OK(ctx, cudaStreamSynchronize(s));
   return B2K_OK;
@@ -903,24 +903,24 @@ int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, unsigned lon
 int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int64_t n, int d, const float* C, int k,
                      int32_t* labels_out, float* mindist_out, bool do_update, bool need_cost, const B2kLoopState* st,
                      cudaStream_t s, const double* prev_counts) {
-  if (plan.variant == 1)
+  if (plan.choice.variant == 1)
     return b2k_launch_fused_t(ctx, plan, X, n, d, C, k, labels_out, mindist_out, do_update,
                               !do_update && (mindist_out != nullptr || need_cost), st, s, prev_counts);
+  const int KP = plan.choice.KP, DP = plan.choice.DP;
   uint8_t* keytab = plan.keytab;
-  k_prep_centers_tc<<<(plan.KP * 32 + 255) / 256, 256, 0, s>>>(C, k, d, plan.KP, plan.DP, plan.c_hi, plan.c_lo,
-                                                               plan.cnorm, st);
-  k_balance_table<<<1, 128, 0, s>>>(do_update ? prev_counts : nullptr, k, plan.KP, keytab, keytab + 256, st);
+  k_prep_centers_tc<<<(KP * 32 + 255) / 256, 256, 0, s>>>(C, k, d, KP, DP, plan.c_hi, plan.c_lo, plan.cnorm, st);
+  k_balance_table<<<1, 128, 0, s>>>(do_update ? prev_counts : nullptr, k, KP, keytab, keytab + 256, st);
   ctx->stats.kernel_launches += 2;
   B2K_CUDA_OK(ctx, cudaGetLastError());
 
   CUtensorMap mx, mh, ml;
-  B2K_TRY(encode_2d(ctx, &mx, X, (uint64_t)d, (uint64_t)n, (uint64_t)d * 4, CHUNK, TM,
-                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
-  const uint32_t cbox = (uint32_t)(plan.pair ? plan.KP / 2 : plan.KP);   // centre rows each CTA keeps in smem
-  B2K_TRY(encode_2d(ctx, &mh, plan.c_hi, (uint64_t)plan.DP, (uint64_t)plan.KP, (uint64_t)plan.DP * 4, CHUNK, cbox,
-                    CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
-  B2K_TRY(encode_2d(ctx, &ml, plan.c_lo, (uint64_t)plan.DP, (uint64_t)plan.KP, (uint64_t)plan.DP * 4, CHUNK, cbox,
-                    CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
+  B2K_TRY(b2k_encode_2d(ctx, &mx, X, (uint64_t)d, (uint64_t)n, (uint64_t)d * 4, CHUNK, TM,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
+  const uint32_t cbox = (uint32_t)(plan.choice.pair ? KP / 2 : KP);   // centre rows each CTA keeps in smem
+  B2K_TRY(b2k_encode_2d(ctx, &mh, plan.c_hi, (uint64_t)DP, (uint64_t)KP, (uint64_t)DP * 4, CHUNK, cbox,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
+  B2K_TRY(b2k_encode_2d(ctx, &ml, plan.c_lo, (uint64_t)DP, (uint64_t)KP, (uint64_t)DP * 4, CHUNK, cbox,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
 
   FusedArgs a{};
   a.n = n;
@@ -939,21 +939,7 @@ int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int
   a.need_cost = (!do_update || mindist_out != nullptr) ? 1 : 0;
   a.st = st;
 
-  int rc = B2K_ERR_UNSUPPORTED;
-#define B2K_DISPATCH(KP_, DP_) \
-  if (!plan.pair && plan.KP == KP_ && plan.DP == DP_) rc = launch_inst<KP_, DP_, false>(ctx, plan.grid, mx, mh, ml, a, s);
-  if (plan.pair && plan.KP == 64 && plan.DP == 128) rc = launch_inst<64, 128, true>(ctx, plan.grid, mx, mh, ml, a, s);
-  B2K_DISPATCH(64, 64)
-  B2K_DISPATCH(64, 32)
-  B2K_DISPATCH(32, 128)
-  B2K_DISPATCH(128, 128)
-  B2K_DISPATCH(128, 64)
-  B2K_DISPATCH(16, 32)
-  B2K_DISPATCH(16, 64)
-  B2K_DISPATCH(32, 64)
-  B2K_DISPATCH(32, 32)
-  B2K_DISPATCH(16, 128)
-#undef B2K_DISPATCH
+  const int rc = launch_listed(Insts{}, KP, DP, ctx, plan.grid, mx, mh, ml, a, s);
   if (rc == B2K_ERR_UNSUPPORTED) return b2k_fail(ctx, rc, "fused kernel: instantiation missing");
   B2K_TRY(rc);
   ctx->stats.kernel_launches++;

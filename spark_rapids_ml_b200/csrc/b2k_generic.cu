@@ -1,7 +1,7 @@
 // Generic (any k, d) SIMT kernels of the Lloyd loop: exact-fp32 tiled assign, ownership-based
 // (atomic-free, deterministic) per-cluster partial sums, fixed-order reductions, finalize.
-// These serve every shape the tcgen05 fused kernel (b2k_fused_tc.cu) does not cover, the k-means||
-// initialiser, and KMeansModel.transform for odd shapes.  sm_100a only; no CPU fallback.
+// These serve every pass b2k_choose_kernel (b2k_api.cu) leaves on the generic path, the update of a chunked Lloyd
+// loop, the k-means|| initialiser, and KMeansModel.transform for odd shapes.  sm_100a only; no CPU fallback.
 //
 // Semantics restated from the reference's backend (EXTERNAL cuML 25.12, called at
 // spark_rapids_ml/clustering.py:383-415): argmin over ||c||^2 - 2 x.c with lowest index on ties,
@@ -263,11 +263,7 @@ UpdatePlan plan_update(const b2k_ctx* ctx, int64_t n, int d, int k) {
 }
 }  // namespace
 
-size_t b2k_update_generic_scratch(b2k_ctx* ctx, int64_t n, int d, int k, int* P_out) {
-  UpdatePlan u = plan_update(ctx, n, d, k);
-  if (P_out) *P_out = u.P;
-  return (size_t)u.P * k * d * sizeof(float) + (size_t)u.P * k * sizeof(int32_t);
-}
+int b2k_update_generic_slots(b2k_ctx* ctx, int64_t n, int d, int k) { return plan_update(ctx, n, d, k).P; }
 
 int b2k_launch_update_generic(b2k_ctx* ctx, const float* X, int64_t n, int d, const int32_t* labels, int k,
                               int P, float* partials, int32_t* counts, const B2kLoopState* st,
@@ -457,21 +453,6 @@ int b2k_launch_gather_rows(b2k_ctx* ctx, const float* X, int d, const int64_t* r
                            int64_t out_row0, cudaStream_t s) {
   if (m <= 0) return B2K_OK;
   k_gather_rows<<<m, 128, 0, s>>>(X, d, rows_local, m, out, out_row0);
-  ctx->stats.kernel_launches++;
-  B2K_CUDA_OK(ctx, cudaGetLastError());
-  return B2K_OK;
-}
-
-__global__ void k_min_inplace(float* __restrict__ a, const float* __restrict__ b, int64_t n) {
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (; i < n; i += stride) a[i] = fminf(a[i], b[i]);
-}
-int b2k_launch_min_inplace(b2k_ctx* ctx, float* a, const float* b, int64_t n, cudaStream_t s) {
-  if (n <= 0) return B2K_OK;
-  int64_t blocks = (n + 255) / 256;
-  if (blocks > ctx->sm_count * 16) blocks = ctx->sm_count * 16;
-  k_min_inplace<<<(unsigned)blocks, 256, 0, s>>>(a, b, n);
   ctx->stats.kernel_launches++;
   B2K_CUDA_OK(ctx, cudaGetLastError());
   return B2K_OK;

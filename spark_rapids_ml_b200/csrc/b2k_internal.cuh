@@ -42,7 +42,6 @@ struct b2k_ctx {
   int check_every = 4;
   int adaptive_path = 1;         // option "adaptive_path": a Lloyd loop on the large-shape kernel falls back to the generic
                                  // kernels for its remaining iterations when most rows need the exact fix-up
-  int force_variant_t = 0;       // option "variant_t": route every supported shape through b2k_fused_t.cu (tests)
   int collect_recheck = 0;       // option "collect_recheck": fill stats.recheck_* (costs a stream sync per call)
   void* xnorm_cache = nullptr;   // float2 [xnorm_cache_rows]: row norms shared by the passes of one fit (B2kNormScope)
   int64_t xnorm_cache_rows = 0;
@@ -150,8 +149,8 @@ int b2k_launch_center_norms(b2k_ctx* ctx, const float* C, int k, int d, float* c
 int b2k_launch_assign_generic(b2k_ctx* ctx, const float* X, int64_t n, int d, const float* C,
                               const float* cnorm, int k, int32_t* labels, float* mindist,
                               const B2kLoopState* st, cudaStream_t s);
-// per-cluster partial sums from labels: partials [P][k*d] f32, counts [P][k] i32; returns P via *P_out.
-size_t b2k_update_generic_scratch(b2k_ctx* ctx, int64_t n, int d, int k, int* P_out);
+// per-cluster partial sums from labels: partials [P][k*d] f32, counts [P][k] i32; b2k_update_generic_slots returns P.
+int b2k_update_generic_slots(b2k_ctx* ctx, int64_t n, int d, int k);
 int b2k_launch_update_generic(b2k_ctx* ctx, const float* X, int64_t n, int d, const int32_t* labels, int k,
                               int P, float* partials, int32_t* counts, const B2kLoopState* st,
                               cudaStream_t s);
@@ -169,7 +168,6 @@ int b2k_launch_fold_f64(b2k_ctx* ctx, const double* in, int m, double* out /*1*/
 int b2k_launch_gather_rows(b2k_ctx* ctx, const float* X, int d, const int64_t* rows_local, int m,
                            float* out, int64_t out_row0, cudaStream_t s);
 // k-means|| helpers
-int b2k_launch_min_inplace(b2k_ctx* ctx, float* a, const float* b, int64_t n, cudaStream_t s);
 int b2k_launch_bernoulli_pick(b2k_ctx* ctx, const float* mind, int64_t n, int64_t row_offset,
                               double scale /* l/phi */, uint64_t seed, int round, int64_t* picked,
                               int* n_picked, int cap, cudaStream_t s);
@@ -180,14 +178,38 @@ int b2k_launch_weighted_update(b2k_ctx* ctx, const float* P, const double* w, co
 int b2k_launch_pairwise_sqdist(b2k_ctx* ctx, const float* P, int M, int d, float* D2, cudaStream_t s);
 
 // ------------------------------------------------------------------------------------------------
+// Which kernels one pass over X runs — b2k_choose_kernel (b2k_api.cu)
+// ------------------------------------------------------------------------------------------------
+// Largest k and d of the 1xTF32 screening kernel (variant 1, b2k_fused_t.cu).
+constexpr int kFusedTMaxK = 256;
+constexpr int kFusedTMaxD = 256;
+// The one 3xTF32 instantiation that runs on CTA pairs (tcgen05 cta_group::2).
+constexpr bool b2k_tc_pair(int KP, int DP) { return KP == 64 && DP == 128; }
+
+struct B2kChoice {
+  enum Kind { GENERIC, FUSED, CHUNKED };
+  Kind kind = GENERIC;
+  int ch = 0;                // CHUNKED: centres per chunk; the fields below then describe the kernel of one chunk
+  int variant = 0;           // 0: b2k_fused_tc.cu (3xTF32); 1: b2k_fused_t.cu (1xTF32 screening + exact recheck)
+  int KP = 0, DP = 0;        // padded cluster count / dimension of the instantiation
+  int pair = 0;              // 1: runs on CTA pairs (tcgen05 cta_group::2), the grid is even
+  int path() const { return kind == GENERIC ? B2K_PATH_GENERIC : B2K_PATH_TCGEN05; }
+};
+// Chooses the kernels of one pass over X[n, d] against k centres under kernel path `path` (B2K_PATH_*); `near_tie`: the
+// caller expects near-ties.  Fails with B2K_ERR_UNSUPPORTED when path = tcgen05 cannot be honoured.
+int b2k_choose_kernel(b2k_ctx* ctx, int path, bool near_tie, int64_t n, int d, int k, const float* X, B2kChoice* out);
+
+// ------------------------------------------------------------------------------------------------
 // tcgen05 fused kernel — b2k_fused_tc.cu
 // ------------------------------------------------------------------------------------------------
+// The smallest 3xTF32 instantiation for (d, k): DP = d rounded up to a multiple of 32 (96 -> 128) and KP >= k.
+// Returns false when none is compiled.
+bool b2k_fused_tc_inst(int d, int k, int* KP, int* DP);
+
 struct B2kFusedPlan {
-  int KP = 0, DP = 0;        // padded cluster count / dimension of the instantiation, 0 = unsupported
+  B2kChoice choice;          // the kernel of the pass (of each chunk, for a chunked pass)
   int grid = 0;              // persistent CTAs
-  int pair = 0;              // 1: CTA-pair (tcgen05 cta_group::2) instantiation, grid is even
-  int variant = 0;           // 0: b2k_fused_tc.cu (k <= 128, d <= 128, 3xTF32); 1: b2k_fused_t.cu (k, d <= 256, 1xTF32 + recheck)
-  int P = 0;                 // partial-sum slots the pass writes (variant 0: grid; variant 1: CTA pairs + 1 for the deferred rows)
+  int P = 0;                 // partial-sum slots the pass writes (variant 0: grid; variant 1: CTA pairs + 4 for the deferred rows)
   int Pc = 0;                // cost partials the pass writes (variant 0: grid; variant 1: grid + fix-up CTAs)
   // scratch carved by b2k_fused_plan (null when planned on a measuring arena)
   float* partials = nullptr;         // [P][k*d] partial sums, [P][k] counts, [Pc] cost: b2k_launch_reduce_partials
@@ -206,9 +228,9 @@ struct B2kFusedPlan {
   int32_t* fix_count = nullptr;      // variant 1: entries per segment
   int seg_cap = 0, mask_cap = 0;
 };
-bool b2k_fused_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X);
-// Plans a fused pass over X[n, d] against k centres and carves its scratch from A.
-int b2k_fused_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan);
+// Plans a fused pass over X[n, d] against k centres on the kernel `c` names (grid, partial slots) and carves its
+// scratch from A.
+int b2k_fused_plan(b2k_ctx* ctx, const B2kChoice& c, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan);
 // Once per fit / lloyd / assign call, before the first b2k_launch_fused on this X (variant 1: row norms, into the plan's
 // scratch or, with a norm scope, into the fit's cache; variant 0: no-op)
 int b2k_fused_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
@@ -223,8 +245,11 @@ int b2k_launch_fused(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, int
 // variant 1 diagnostics: {rows re-decided exactly, candidate distances evaluated} since the last b2k_fused_prepare
 int b2k_fused_recheck_stats(b2k_ctx* ctx, const B2kFusedPlan& plan, unsigned long long out[2], cudaStream_t s);
 
+// Tensor map of a row-major f32 matrix [outer][inner] with 128B swizzle (both fused kernels).
+int b2k_encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,
+                  uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer, CUtensorMapL2promotion l2);
+
 // b2k_fused_t.cu (variant 1)
-bool b2k_fused_t_supported(const b2k_ctx* ctx, int64_t n, int d, int k, const float* X);
 int b2k_fused_t_plan(b2k_ctx* ctx, int64_t n, int d, int k, Arena& A, B2kFusedPlan* plan);
 int b2k_fused_t_prepare(b2k_ctx* ctx, B2kFusedPlan& plan, const float* X, int64_t n, int d, B2kNormScope* norms,
                         cudaStream_t s);
@@ -233,8 +258,6 @@ int b2k_launch_fused_t(b2k_ctx* ctx, const B2kFusedPlan& plan, const float* X, i
                        cudaStream_t s, const double* prev_counts);
 int b2k_launch_merge_chunk(b2k_ctx* ctx, float* md_acc, int32_t* lab_acc, const float* md, const int32_t* lab, int base,
                            int64_t n, const B2kLoopState* st, cudaStream_t s);
-int b2k_fused_encode_2d(b2k_ctx* ctx, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,
-                        uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer, int l2_256);
 
 // ------------------------------------------------------------------------------------------------
 // comm — b2k_comm.cu

@@ -2,8 +2,7 @@
 tcgen05 1xTF32 screening + proven-bound exact recheck, through the C ABI, against the fp64 oracle.
 
 Parity rule as in test_gpu_parity.py: labels bit-exact except rows whose fp64 margin is below 1e-6;
-centroids within 1e-4 relative.  Shapes the 3xTF32 kernel covers are pushed through this kernel with option
-"variant_t" so that both instantiations (DP = 128 and DP = 256) are exercised.
+centroids within 1e-4 relative.
 """
 import numpy as np
 import pytest
@@ -32,30 +31,26 @@ def _dev(x):
     return torch.from_numpy(np.ascontiguousarray(x)).cuda()
 
 
-@pytest.mark.parametrize("n,d,k,gen,force", [
-    (128, 256, 256, "blobs", 0),
-    (20000, 256, 256, "blobs", 0),       # BASELINE cfg3's (k, d)
-    (5000, 256, 256, "uniform", 0),      # near-tie stress: about half of the rows take the exact recheck
-    (3001, 256, 200, "blobs", 0),        # ragged last step, k < 256 (padding clusters)
-    (4096, 192, 130, "uniform", 0),      # d not a multiple of 256: TMA zero fill
-    (1000, 256, 64, "blobs", 0),         # k <= 128 with d > 128: the peer CTA holds only padding clusters
-    (777, 132, 256, "uniform", 0),       # d % 32 != 0
-    (64, 256, 256, "uniform", 0),        # fewer rows than clusters, half a step
-    (1, 256, 3, "uniform", 0),           # single row
-    (5000, 128, 64, "uniform", 1),       # DP = 128 instantiation (forced: the 3xTF32 kernel would take these)
-    (3000, 100, 40, "blobs", 1),
+@pytest.mark.parametrize("n,d,k,gen", [
+    (128, 256, 256, "blobs"),
+    (20000, 256, 256, "blobs"),          # BASELINE cfg3's (k, d)
+    (5000, 256, 256, "uniform"),         # near-tie stress: about half of the rows take the exact recheck
+    (3001, 256, 200, "blobs"),           # ragged last step, k < 256 (padding clusters)
+    (4096, 192, 130, "uniform"),         # d not a multiple of 256: TMA zero fill
+    (1000, 256, 64, "blobs"),            # k <= 128 with d > 128: the peer CTA holds only padding clusters
+    (777, 132, 256, "uniform"),          # d % 32 != 0
+    (64, 256, 256, "uniform"),           # fewer rows than clusters, half a step
+    (1, 256, 3, "uniform"),              # single row
+    (5000, 128, 200, "uniform"),         # DP = 128 instantiation (k > 128)
+    (3000, 20, 100, "blobs"),            # DP = 128, d % 32 != 0, the peer CTA holds only padding clusters
 ])
-def test_assign_large_matches_oracle(ctx, n, d, k, gen, force):
+def test_assign_large_matches_oracle(ctx, n, d, k, gen):
     X = ko.make_blobs(n, d, k, seed=7)[0] if gen == "blobs" else ko.make_uniform(n, d, seed=7)
     rng = np.random.default_rng(3)
     C = X[rng.choice(n, size=k, replace=(n < k))].copy() + (0.01 if gen == "uniform" else 0.0)
-    ctx.set_option("variant_t", force)
-    try:
-        ctx.reset_stats()
-        labels, md = ctx.kmeans_assign(_dev(X), _dev(C), want_mindist=True)
-        st = ctx.stats()
-    finally:
-        ctx.set_option("variant_t", 0)
+    ctx.reset_stats()
+    labels, md = ctx.kmeans_assign(_dev(X), _dev(C), want_mindist=True)
+    st = ctx.stats()
     assert st["last_path"] == 2 and st["fused_tc_launches"] >= 1
     cmp = ko.compare_labels(X, C, labels.cpu().numpy(), tau=TAU)
     assert cmp["n_mismatch_outside_margin"] == 0, cmp
@@ -83,13 +78,13 @@ def test_large_tie_break_and_duplicates(ctx):
     assert int((labels == 9).sum()) == 0
 
 
-@pytest.mark.parametrize("n,d,k,iters,gen,force", [
-    (20000, 256, 256, 4, "blobs", 0),
-    (6000, 256, 256, 3, "uniform", 0),
-    (30000, 128, 64, 4, "blobs", 1),
-    (5000, 160, 200, 3, "blobs", 0),
+@pytest.mark.parametrize("n,d,k,iters,gen", [
+    (20000, 256, 256, 4, "blobs"),
+    (6000, 256, 256, 3, "uniform"),
+    (30000, 128, 160, 4, "blobs"),
+    (5000, 160, 200, 3, "blobs"),
 ])
-def test_lloyd_large_matches_oracle(ctx, n, d, k, iters, gen, force):
+def test_lloyd_large_matches_oracle(ctx, n, d, k, iters, gen):
     X, ctr = ko.make_blobs(n, d, k, seed=11)
     if gen == "uniform":
         X = ko.make_uniform(n, d, seed=11)
@@ -97,12 +92,8 @@ def test_lloyd_large_matches_oracle(ctx, n, d, k, iters, gen, force):
     else:
         C0 = (ctr + 0.25 * np.random.default_rng(0).normal(size=ctr.shape)).astype(np.float32)
     ref = ko.lloyd([X], C0, iters, -1.0)
-    ctx.set_option("variant_t", force)
-    try:
-        C = _dev(C0)
-        n_it, _ = ctx.kmeans_lloyd(_dev(X), C, iters, -1.0)
-    finally:
-        ctx.set_option("variant_t", 0)
+    C = _dev(C0)
+    n_it, _ = ctx.kmeans_lloyd(_dev(X), C, iters, -1.0)
     assert n_it == iters and ctx.stats()["last_path"] == 2
     # an admissible (< 1e-6 margin) tie row may send two trajectories apart on uniform data: check one exact step too
     lab0, _, margin0 = ko.assign(X, C0)
@@ -257,6 +248,56 @@ def test_assign_and_lloyd_beyond_256_clusters_run_in_chunks(n, d, k, gen):
         lg, _ = c.kmeans_assign(_dev(X), _dev(C0))
         assert c.stats()["last_path"] == 1
         assert ko.compare_labels(X, C0, lg.cpu().numpy(), tau=TAU)["n_mismatch_outside_margin"] == 0
+    finally:
+        c.close()
+
+
+# Deltas of (kernel_launches, fused_tc_launches, generic_launches) and last_path of one assign pass without min distances,
+# or None where kernel_path = tcgen05 must fail.  Per pass: 3 kernels on the 3xTF32 kernel (centre split, update table,
+# pass), 5 on the screening kernel (row norms, centre prep, tables, pass, deferred-row labels) and 2 on the generic path
+# (centre norms, assign); a chunked pass runs the row norms once, one fused pass per chunk and a merge for every chunk
+# after the first.
+@pytest.mark.parametrize("d,k,path,misaligned,expect", [
+    (64, 32, 0, False, (3, 1, 0, 2)),        # 3xTF32 <32, 64>
+    (128, 64, 0, False, (3, 1, 0, 2)),       # 3xTF32 <64, 128> on CTA pairs
+    (32, 64, 0, False, (3, 1, 0, 2)),        # 3xTF32 <64, 32>
+    (32, 100, 0, False, (5, 1, 0, 2)),       # d <= 32, 64 < k <= 128: no <128, 32>, the screening kernel at DP = 128
+    (128, 200, 0, False, (5, 1, 0, 2)),      # screening kernel, DP = 128
+    (256, 256, 0, False, (5, 1, 0, 2)),      # screening kernel, DP = 256
+    (6, 16, 0, False, (2, 0, 1, 1)),         # d % 4 != 0: no TMA
+    (6, 16, 2, False, None),
+    (260, 16, 0, False, (2, 0, 1, 1)),       # d > 256
+    (260, 16, 2, False, None),
+    (64, 32, 0, True, (2, 0, 1, 1)),         # X not 16-byte aligned
+    (64, 32, 1, False, (2, 0, 1, 1)),        # kernel_path = generic
+    (64, 300, 0, False, (11, 3, 0, 2)),      # 3 chunks of 128 on 3xTF32 <128, 64> + 2 merges
+    (200, 600, 0, False, (15, 3, 0, 2)),     # row norms + 3 chunks of 256 on the screening kernel + 2 merges
+    (32, 300, 0, False, (15, 3, 0, 2)),      # d <= 32: chunks of 128 on the screening kernel
+])
+def test_each_shape_takes_its_kernel(d, k, path, misaligned, expect):
+    """The kernel each (d, k) runs on (b2k_choose_kernel in csrc/b2k_api.cu), seen through the public stats."""
+    import torch
+    from spark_rapids_ml_b200 import _native
+
+    n = 4096
+    X = torch.from_numpy(ko.make_uniform(n, d, seed=2)).cuda()
+    if misaligned:   # a contiguous view starting 4 bytes into its buffer
+        X = torch.empty(n * d + 1, dtype=torch.float32, device="cuda")[1:].view(n, d).copy_(X)
+        assert X.data_ptr() % 16 == 4
+    C = X[:k].clone()
+    c = _native.Context(0)
+    try:
+        c.set_option("kernel_path", path)
+        if expect is None:
+            with pytest.raises(_native.B2KError) as e:
+                c.kmeans_assign(X, C)
+            assert e.value.code == 4   # B2K_ERR_UNSUPPORTED
+            return
+        b = c.stats()
+        c.kmeans_assign(X, C)
+        a = c.stats()
+        got = tuple(a[f] - b[f] for f in ("kernel_launches", "fused_tc_launches", "generic_launches"))
+        assert got + (a["last_path"],) == expect
     finally:
         c.close()
 
